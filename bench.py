@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W                # this repository (B200 kernels)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # also write the last timed step's results
 
 One step = one ``recognize`` pass over a batch of 32 synthetic pages (768x768 RGB, 32 rendered
 words each, ``Pipeline(scale=2)`` -> 32x1536x1536 detector input, BASELINE.json configs[3]); with
@@ -16,6 +17,9 @@ Timed region: K steps bracketed by barrier + cuda synchronize, CUDA events, max 
 ``roofline``: the dominant kernel (tcgen05 conv) -- algorithmic FLOPs of its launches in one step
              / their CUDA-event time, against the measured bf16 peak (MEASURED_PEAKS.json).
 ``cpu_baseline``: the oracle port of the reference path on the host cores, bounded sample.
+
+``--dump-outputs DIR`` writes what the last timed step of ``value`` returned (``dump_outputs``).  Pages and weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -76,6 +80,33 @@ def words_read(result, words, rects):
                 found.add(inside[0])
         hit += len(found)
     return hit, sum(len(w) for w in words)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(result, out_dir):
+    """Writes a ``recognize`` result (per image, a list of (text, box)) as float32 arrays, images and words in order:
+
+    ``counts.npy`` (n_images,)          words found in each image
+    ``boxes.npy``  (n_words, 4, 2)      word quads in source-image pixels
+    ``texts.npy``  (n_words, max_len)   Unicode code points of each word's text, zero-padded
+    """
+    texts = [text for group in result for text, _ in group]
+    codes = np.zeros((len(texts), max((len(t) for t in texts), default=0)), np.float32)
+    for i, text in enumerate(texts):
+        codes[i, :len(text)] = [ord(c) for c in text]
+    arrays = {
+        "counts": np.array([len(group) for group in result], np.float32),
+        "boxes": np.array([box for group in result for _, box in group], np.float32).reshape(-1, 4, 2),
+        "texts": codes,
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"outputs of one step take {total} bytes, more than the {DUMP_LIMIT_BYTES} a dump may hold")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -240,6 +271,7 @@ def run_b200(args):
             result = D.recognize_sharded(pipe, inputs, max_boxes=max_boxes, presharded=True)
         if result is not None:
             stats["words"] = sum(len(g) for g in result)
+            stats["last"] = result
         return result
 
     def barrier():
@@ -263,6 +295,7 @@ def run_b200(args):
             result = stream.flush()
             if result is not None:
                 stats["words"] = sum(len(g) for g in result)
+                stats["last"] = result
         else:
             for _ in range(steps):
                 step(inputs)
@@ -285,7 +318,9 @@ def run_b200(args):
         sampler.start()
     launches0 = det.ctx.launch_count() + rec.ctx.launch_count()
     D.stats["decode_ms"], D.stats["decodes"] = 0.0, 0
+    stats["last"] = None
     ms_dev = timed(pages_dev, args.steps)
+    last_result = stats["last"]                          # what the last timed step returned (rank 0)
     per_rank_dev = stats.get("per_rank_ms")
     decode_ms = D.stats["decode_ms"] / max(D.stats["decodes"], 1)
     launches = det.ctx.launch_count() + rec.ctx.launch_count() - launches0
@@ -350,6 +385,8 @@ def run_b200(args):
         v, desc, cores = cpu_sample(host_threads(), 1)
         line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
                                 "sample": "oracle port of the reference path (TensorFlow not installable offline): " + desc}
+    if args.dump_outputs:
+        dump_outputs(last_result, args.dump_outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -362,7 +399,13 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results to DIR/<name>.npy (b200 only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     sys.exit(run_reference(args) if args.impl == "reference" else run_b200(args))
 
 

@@ -4,9 +4,9 @@ prediction, ``"eventdock"``; a blank image -> no prediction.
 
 Neither weight file exists offline (no network, SURVEY.md 8(c)), so the test SKIPS unless they are present in the
 keras-ocr cache directory (``~/.keras-ocr`` or ``$KERAS_OCR_CACHE_DIR``, reference tools.py:495-498) with the reference's
-sha256 digests (detection.py:647-658, recognition.py:27-44), and unless the reference's test image can be found
-(``$KERAS_OCR_TEST_IMAGE``, or the reference checkout).  Everything between the files and the assertion is the product
-path: ``weights.load_craft_pth`` (torch.load), ``hdf5.read_datasets`` (own HDF5 reader), the CUDA pipeline."""
+sha256 digests (detection.py:647-658, recognition.py:27-44).  The reference's test image is stored as
+``tests/golden/test_image.jpg``.  Everything between the files and the assertion is the product path:
+``weights.load_craft_pth`` (torch.load), ``hdf5.read_datasets`` (own HDF5 reader), the CUDA pipeline."""
 import os
 
 import numpy as np
@@ -20,22 +20,12 @@ CRAFT = ("craft_mlt_25k.pth", "4a5efbfb48b4081100544e75e1e2b57f8de3d84f213004b14
 CRNN = ("crnn_kurapan.h5", "a7d8086ac8f5c3d6a0a828f7d6fbabcaf815415dd125c32533013f85603be46d")
 
 
-def _test_image():
-    for path in (os.environ.get("KERAS_OCR_TEST_IMAGE"), "/root/reference/tests/test_image.jpg",
-                 os.path.join(os.path.dirname(__file__), "golden", "test_image.jpg")):
-        if path and os.path.isfile(path):
-            return path
-    return None
-
-
-def test_pipeline_known_answer_eventdock(cuda_device):
+def test_pipeline_known_answer_eventdock(cuda_device, golden_dir):
     cache = tools.get_default_cache_dir()
     missing = [name for name, _ in (CRAFT, CRNN) if not os.path.isfile(os.path.join(cache, name))]
     if missing:
         pytest.skip(f"pretrained weights not in {cache}: {', '.join(missing)} (no network to download them)")
-    image_path = _test_image()
-    if image_path is None:
-        pytest.skip("reference tests/test_image.jpg not found (set KERAS_OCR_TEST_IMAGE)")
+    image_path = os.path.join(golden_dir, "test_image.jpg")
     for name, digest in (CRAFT, CRNN):
         assert tools.sha256sum(os.path.join(cache, name)) == digest, f"{name}: sha256 mismatch"
 

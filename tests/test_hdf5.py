@@ -35,17 +35,14 @@ def test_round_trip_groups_contiguous_and_chunked(tmp_path):
         hdf5.read_datasets(b"not an hdf5 file at all" * 100)
 
 
-def test_reads_a_file_written_by_the_hdf5_c_library():
-    """The only real HDF5 file in this image: scipy's MATLAB v7.3 fixture (HDF5 1.8 C library, 512-byte user block,
-    object-header continuation blocks).  Its twin in MATLAB's own v7 format, read by scipy, holds the same variable."""
+def test_reads_a_file_written_by_the_hdf5_c_library(golden_dir):
+    """A real HDF5 file: scipy's MATLAB v7.3 test fixture, stored in tests/golden (HDF5 1.8 C library, 512-byte user
+    block, object-header continuation blocks).  Its twin in MATLAB's own v7 format, read by scipy, holds the same
+    variable."""
     import scipy.io
-    data = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data")
-    h5 = os.path.join(data, "testhdf5_7.4_GLNX86.mat")
-    if not os.path.exists(h5):
-        pytest.skip("scipy test data not installed")
-    got = hdf5.read_datasets(h5)
+    got = hdf5.read_datasets(os.path.join(golden_dir, "testhdf5_7.4_GLNX86.mat"))
     assert list(got) == ["testdouble"] and got["testdouble"].dtype == np.float64
-    twin = scipy.io.loadmat(os.path.join(data, "testdouble_7.4_GLNX86.mat"))["testdouble"]
+    twin = scipy.io.loadmat(os.path.join(golden_dir, "testdouble_7.4_GLNX86.mat"))["testdouble"]
     assert np.array_equal(got["testdouble"].ravel(), twin.ravel())
 
 
