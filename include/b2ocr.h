@@ -75,6 +75,19 @@ int b2o_profile_read(b2o_ctx* ctx, double* tc_ms, double* tc_flop, int64_t* tc_l
 int b2o_load_craft(b2o_ctx* ctx, const b2o_tensor* tensors, int n);
 int b2o_load_crnn(b2o_ctx* ctx, const b2o_tensor* tensors, int n);
 
+/* Crop geometry of the recognizer, build_model(height, width, rnn_steps_to_discard) (recognition.py:13-23, 214, 328).
+ * Crops are height x width; the conv stack's two floor-ing 2x2 max pools leave T = width / 4 time steps of
+ * Hf = height / 4 feature rows, so fc_9.kernel is (Hf*512, 128) and stn.dense_a.kernel (T*Hf*32, 64); label rows are
+ * T - rnn_steps_to_discard long.  Call it BEFORE b2o_load_crnn, which checks those shapes against it (B2O_ERR_STATE
+ * once a CRNN is loaded).  Default 31 x 200, 2 discarded: T = 50, 48-long label rows.  Supported: height 16..64,
+ * width 32..800, 0 <= rnn_steps_to_discard < width / 4 (B2O_ERR_ARG otherwise).  The warp, crop-to-input, forward,
+ * workspace and tap entry points below follow the context's geometry.                                           */
+#define B2O_CRNN_MIN_HEIGHT 16
+#define B2O_CRNN_MAX_HEIGHT 64
+#define B2O_CRNN_MIN_WIDTH 32
+#define B2O_CRNN_MAX_WIDTH 800
+int b2o_set_crnn_geometry(b2o_ctx* ctx, int height, int width, int rnn_steps_to_discard);
+
 /* tools.resize_image + tools.pad (tools.py:378-398, 356-375; pipeline.py:44-57), one image:
  * bilinear (OpenCV fixed-point INTER_LINEAR) resize of src (hs x ws x 3) to (hr x wr), written into
  * the top-left of dst image `index` of a (n, hp, wp, 3) batch; the rest is filled with 255.   */
@@ -127,26 +140,31 @@ int b2o_compact_boxes(b2o_ctx* ctx, const float* boxes_dev, const int32_t* count
                       float* flat_dev, int32_t* image_index_dev, void* stream);
 
 /* tools.warpBox over box groups (recognition.py:506-519; tools.py:61-117).  boxes: (n_boxes,4,2)
- * float32; image_index[k] selects the gray image of box k.  crops: (n_boxes,31,200) uint8
- * (exactly warpBox's output) and, when crnn_in != NULL, the CRNN input (n_boxes,200,31) fp16 =
- * crop/255 after Permute((2,1,3)) and the axis flip of recognition.py:215-216.                */
+ * float32; image_index[k] selects the gray image of box k.  crops: (n_boxes,height,width) uint8
+ * (exactly warpBox's output at the context's crop size, 31 x 200 by default) and, when crnn_in != NULL, the
+ * CRNN input (n_boxes,width,height) fp16 = crop/255 after Permute((2,1,3)) and the axis flip of
+ * recognition.py:215-216.                                                                      */
 int b2o_warp_boxes(b2o_ctx* ctx, const uint8_t* gray_dev, int n, int h, int w,
                    const float* boxes_dev, const int32_t* image_index_dev, int n_boxes,
                    uint8_t* crops_dev, void* crnn_in_dev, void* stream);
 
 /* The same for a recognizer built with color=True (recognition.py:214, 508-510: crops are cut from the RGB image, no
- * gray conversion): rgb (n,h,w,3) uint8, crops (n_boxes,31,200,3) uint8, crnn_in (n_boxes,200,31,3) fp16.            */
+ * gray conversion): rgb (n,h,w,3) uint8, crops (n_boxes,height,width,3) uint8, crnn_in (n_boxes,width,height,3) fp16. */
 int b2o_warp_boxes_color(b2o_ctx* ctx, const uint8_t* rgb_dev, int n, int h, int w,
                          const float* boxes_dev, const int32_t* image_index_dev, int n_boxes,
                          uint8_t* crops_dev, void* crnn_in_dev, void* stream);
 
 /* prediction_model.predict (recognition.py:535; graph 214-333): CRNN + STN + BiLSTM + greedy CTC.
- * crnn_in: (b,200,31) fp16 from b2o_warp_boxes (or b2o_crops_to_input).  labels: (b,48) int32,
- * merged + blank-free, padded with -1 -- the tensor recognize_from_boxes iterates (527-534).  */
+ * crnn_in: (b,width,height) fp16 from b2o_warp_boxes (or b2o_crops_to_input).  labels: (b,T-discard) int32
+ * ((b,48) at the default geometry), merged + blank-free, padded with -1 -- the tensor recognize_from_boxes
+ * iterates (527-534).  b2o_crnn_workspace_bytes has no context and sizes the default 31 x 200 geometry;
+ * b2o_crnn_workspace_bytes_for sizes the context's.                                                          */
 size_t b2o_crnn_workspace_bytes(int b);
+size_t b2o_crnn_workspace_bytes_for(const b2o_ctx* ctx, int b);
+/* crops (b,height,width) uint8 -> (b,width,height) fp16 (the layout b2o_warp_boxes writes to crnn_in).        */
 int b2o_crops_to_input(b2o_ctx* ctx, const uint8_t* crops_dev, int b, void* crnn_in_dev, void* stream);
-/* crops (b,31,200,3) uint8 -> (b,200,31,3) fp16 for a color=True recognizer (conv_1.kernel of shape (3,3,3,64));
- * b2o_crnn_forward then takes that 3-channel input.                                                              */
+/* crops (b,height,width,3) uint8 -> (b,width,height,3) fp16 for a color=True recognizer (conv_1.kernel of shape
+ * (3,3,3,64)); b2o_crnn_forward then takes that 3-channel input.                                              */
 int b2o_crops_to_input_color(b2o_ctx* ctx, const uint8_t* crops_dev, int b, void* crnn_in_dev, void* stream);
 int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in_dev, int b, int32_t* labels_dev,
                      void* ws_dev, size_t ws_bytes, void* stream);
@@ -156,17 +174,26 @@ int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in_dev, int b, int32_t* labe
  * tools.py:232-260)][rec_boxes x 48 labels as int8, -1 padded], b2o_record_floats(rec_boxes) floats long.
  * boxes/counts as written by b2o_get_boxes, labels (sum counts, 48) int32 as written by b2o_crnn_forward
  * (NULL when no image has a box).  Rows n..rows-1 (a short last shard) get count -1.  The class count
- * must fit int8 (alphabets up to 126 characters).                                               */
+ * must fit int8 (alphabets up to 126 characters).
+ * The *_steps forms take the label row length of a recognizer with another crop geometry (T - discard, see
+ * b2o_set_crnn_geometry): labels (sum counts, steps) int32; the label area then holds rec_boxes * steps int8 back
+ * to back in rec_boxes * ceil(steps / 4) floats, the unused tail bytes -1.  b2o_record_floats and b2o_pack_records
+ * are the forms with steps = 48.                                                                 */
 size_t b2o_record_floats(int rec_boxes);
+size_t b2o_record_floats_steps(int rec_boxes, int steps);
 int b2o_pack_records(b2o_ctx* ctx, const float* boxes_dev, const int32_t* counts_dev, const int32_t* labels_dev,
                      const float* inv_scale_dev, int n, int max_boxes, int rows, int rec_boxes,
                      float* records_dev, void* stream);
+int b2o_pack_records_steps(b2o_ctx* ctx, const float* boxes_dev, const int32_t* counts_dev, const int32_t* labels_dev,
+                           const float* inv_scale_dev, int n, int max_boxes, int rows, int rec_boxes, int steps,
+                           float* records_dev, void* stream);
 
 /* Debug / test taps (not on the product path): b2o_set_debug_taps(ctx, 1) makes b2o_crnn_forward also write the
  * fp32 fc_12 outputs ("logits") to its workspace; by default (0) the fused Dense + CTC kernel keeps them in
  * registers and only the labels reach memory.  b2o_crnn_tap copies an intermediate of the last forward pass.
- * b2o_crnn_tap names: "features" (b,50,7,512 f16), "theta" (b,6 f32), "warped" (b,50,7,512 f16),
- * "fc_9" (b,50,128 f16), "l1" (b,50,128 f16), "l2" (b,50,256 f16), "logits" (b,48,K f32).      */
+ * b2o_crnn_tap names: "features" (b,T,Hf,512 f16), "theta" (b,6 f32), "warped" (b,T,Hf,512 f16),
+ * "fc_9" (b,T,128 f16), "l1" (b,T,128 f16), "l2" (b,T,256 f16), "logits" (b,T-discard,K f32); at the default
+ * geometry T = 50, Hf = 7, T-discard = 48 (b2o_set_crnn_geometry).                             */
 int b2o_set_debug_taps(b2o_ctx* ctx, int on);
 int b2o_crnn_tap(b2o_ctx* ctx, const char* name, const void* ws_dev, int b, void* out_dev,
                  size_t out_bytes, void* stream);

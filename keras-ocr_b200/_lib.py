@@ -14,6 +14,8 @@ LIB_PATH = os.environ.get("B2O_LIB") or os.path.join(_HERE, "libb2ocr.so")      
 
 CONV_AUTO, CONV_SIMT, CONV_TC_GENERIC = 0, 1, 2
 MAX_CLASSES = 1024            # B2O_MAX_CLASSES in include/b2ocr.h
+CRNN_HEIGHTS = (16, 64)       # B2O_CRNN_MIN_HEIGHT / B2O_CRNN_MAX_HEIGHT: supported recognizer crop heights
+CRNN_WIDTHS = (32, 800)       # B2O_CRNN_MIN_WIDTH / B2O_CRNN_MAX_WIDTH: ... and widths
 
 
 class B2OError(RuntimeError):
@@ -40,6 +42,7 @@ SIGNATURES = {
     "b2o_profile_read": (_i, [_vp, _c.POINTER(_c.c_double), _c.POINTER(_c.c_double), _c.POINTER(_c.c_int64)]),
     "b2o_load_craft": (_i, [_vp, _c.POINTER(_Tensor), _i]),
     "b2o_load_crnn": (_i, [_vp, _c.POINTER(_Tensor), _i]),
+    "b2o_set_crnn_geometry": (_i, [_vp, _i, _i, _i]),
     "b2o_resize_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "b2o_resize_pad_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp]),
     "b2o_jpeg_info": (_i, [_vp, _vp, _sz, _c.POINTER(_i), _c.POINTER(_i), _c.POINTER(_i)]),
@@ -51,11 +54,14 @@ SIGNATURES = {
     "b2o_get_boxes": (_i, [_vp, _vp, _i, _i, _i, _f, _f, _f, _i, _vp, _vp, _i, _vp, _sz, _vp]),
     "b2o_compact_boxes": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "b2o_record_floats": (_sz, [_i]),
+    "b2o_record_floats_steps": (_sz, [_i, _i]),
     "b2o_pack_records": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp]),
+    "b2o_pack_records_steps": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "b2o_warp_boxes": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "b2o_warp_boxes_color": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "b2o_crops_to_input_color": (_i, [_vp, _vp, _i, _vp, _vp]),
     "b2o_crnn_workspace_bytes": (_sz, [_i]),
+    "b2o_crnn_workspace_bytes_for": (_sz, [_vp, _i]),
     "b2o_crops_to_input": (_i, [_vp, _vp, _i, _vp, _vp]),
     "b2o_crnn_forward": (_i, [_vp, _vp, _i, _vp, _vp, _sz, _vp]),
     "b2o_set_debug_taps": (_i, [_vp, _i]),
@@ -151,6 +157,10 @@ class Context:
         arr, keep = _tensor_array(weights)
         self._check(self.lib.b2o_load_craft(self.handle, arr, len(weights)), "b2o_load_craft")
 
+    def set_crnn_geometry(self, height, width, rnn_steps_to_discard):
+        self._check(self.lib.b2o_set_crnn_geometry(self.handle, int(height), int(width), int(rnn_steps_to_discard)),
+                    "b2o_set_crnn_geometry")
+
     def load_crnn(self, weights):
         arr, keep = _tensor_array(weights)
         self._check(self.lib.b2o_load_crnn(self.handle, arr, len(weights)), "b2o_load_crnn")
@@ -193,19 +203,26 @@ class Context:
         self._check(self.lib.b2o_compact_boxes(self.handle, boxes, counts, n, max_boxes, flat, image_index, stream),
                     "b2o_compact_boxes")
 
-    def record_floats(self, rec_boxes):
-        return int(self.lib.b2o_record_floats(rec_boxes))
+    def record_floats(self, rec_boxes, steps=None):
+        if steps is None:
+            return int(self.lib.b2o_record_floats(rec_boxes))
+        return int(self.lib.b2o_record_floats_steps(rec_boxes, int(steps)))
 
-    def pack_records(self, boxes, counts, labels, inv_scale, n, max_boxes, rows, rec_boxes, records, stream):
-        self._check(self.lib.b2o_pack_records(self.handle, boxes, counts, labels, inv_scale, n, max_boxes, rows,
-                                              rec_boxes, records, stream), "b2o_pack_records")
+    def pack_records(self, boxes, counts, labels, inv_scale, n, max_boxes, rows, rec_boxes, records, stream, steps=None):
+        if steps is None:
+            self._check(self.lib.b2o_pack_records(self.handle, boxes, counts, labels, inv_scale, n, max_boxes, rows,
+                                                  rec_boxes, records, stream), "b2o_pack_records")
+        else:
+            self._check(self.lib.b2o_pack_records_steps(self.handle, boxes, counts, labels, inv_scale, n, max_boxes, rows,
+                                                        rec_boxes, int(steps), records, stream), "b2o_pack_records_steps")
 
     def warp_boxes(self, gray, n, h, w, boxes, image_index, n_boxes, crops, crnn_in, stream, color=False):
         fn = self.lib.b2o_warp_boxes_color if color else self.lib.b2o_warp_boxes
         self._check(fn(self.handle, gray, n, h, w, boxes, image_index, n_boxes, crops, crnn_in, stream), "b2o_warp_boxes")
 
     def crnn_workspace_bytes(self, b):
-        return int(self.lib.b2o_crnn_workspace_bytes(b))
+        """Workspace of b2o_crnn_forward at this context's crop geometry (b2o_crnn_workspace_bytes_for)."""
+        return int(self.lib.b2o_crnn_workspace_bytes_for(self.handle, b))
 
     def crops_to_input(self, crops, b, crnn_in, stream, color=False):
         fn = self.lib.b2o_crops_to_input_color if color else self.lib.b2o_crops_to_input

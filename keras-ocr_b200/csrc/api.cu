@@ -9,12 +9,12 @@
 #include "common.cuh"
 
 int stn_theta_run(b2o_ctx* ctx, const __half* d1, int B, float* theta, cudaStream_t st);
-int stn_col2im_run(b2o_ctx* ctx, const __half* y, const float* bias, int B, __half* out, cudaStream_t st);
-int stn_sample_run(b2o_ctx* ctx, const __half* feat, const float* theta, int B, __half* out, cudaStream_t st);
-int lstm_run(b2o_ctx* ctx, const float* xw, int xw_ld, int xw_off, const __half* u, int B, int backwards, __half* out,
+int stn_col2im_run(b2o_ctx* ctx, const __half* y, const float* bias, int B, int H, int W, __half* out, cudaStream_t st);
+int stn_sample_run(b2o_ctx* ctx, const __half* feat, const float* theta, int B, int Hh, int Ww, __half* out, cudaStream_t st);
+int lstm_run(b2o_ctx* ctx, const float* xw, int xw_ld, int xw_off, const __half* u, int B, int T, int backwards, __half* out,
              int out_ld, int out_off, cudaStream_t st);
 int add_run(b2o_ctx* ctx, const __half* a, const __half* b, __half* o, long long n, cudaStream_t st);
-int fc_ctc_run(b2o_ctx* ctx, const __half* l2, int B, float* logits, int* labels, cudaStream_t st);
+int fc_ctc_run(b2o_ctx* ctx, const __half* l2, int B, int T, int discard, float* logits, int* labels, cudaStream_t st);
 
 namespace {
 
@@ -202,20 +202,23 @@ struct CrnnPlan {
       off_warp, off_fc9, off_xw1, off_hf, off_hb, off_l1, off_xw2, off_l2, off_logits, bytes;
 };
 
-CrnnPlan plan_crnn(int b) {
+// Buffer plan of the CRNN forward pass at crop geometry g (NHWC fp16 unless noted; the conv stack's "h" axis is the
+// crop's width, its "w" axis the crop's height): (W0, H0) = (width, height) -> pooled (W1, H1) -> (T, Hf).
+CrnnPlan plan_crnn(int b, const CrnnGeometry& g) {
   CrnnPlan p;
   p.b = b;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t r = off; off += (bytes + 255) / 256 * 256; return r; };
   const size_t B = static_cast<size_t>(b);
-  p.off_x1 = take(B * 200 * 31 * 64 * 2); p.off_x2 = take(B * 200 * 31 * 128 * 2); p.off_x3 = take(B * 200 * 31 * 256 * 2);
-  p.off_p3 = take(B * 100 * 15 * 256 * 2); p.off_x4 = take(B * 100 * 15 * 256 * 2); p.off_x5 = take(B * 100 * 15 * 512 * 2);
-  p.off_p5 = take(B * 50 * 7 * 512 * 2); p.off_x6 = take(B * 50 * 7 * 512 * 2); p.off_x7 = take(B * 50 * 7 * 512 * 2);
-  p.off_sa = take(B * 50 * 7 * 16 * 2); p.off_sb = take(B * 50 * 7 * 32 * 2); p.off_d1 = take(B * 64 * 2);
-  p.off_theta = take(B * 6 * 4); p.off_warp = take(B * 50 * 7 * 512 * 2); p.off_fc9 = take(B * 50 * 128 * 2);
-  p.off_xw1 = take(B * 50 * 1024 * 4); p.off_hf = take(B * 50 * 128 * 2); p.off_hb = take(B * 50 * 128 * 2);
-  p.off_l1 = take(B * 50 * 128 * 2); p.off_xw2 = take(B * 50 * 1024 * 4); p.off_l2 = take(B * 50 * 256 * 2);
-  p.off_logits = take(B * 48 * B2O_MAX_CLASSES * 4);   // sized for the largest alphabet so the plan is context-free
+  const size_t W0 = g.width, H0 = g.height, W1 = W0 / 2, H1 = H0 / 2, T = g.steps(), Hf = g.feat_h();
+  p.off_x1 = take(B * W0 * H0 * 64 * 2); p.off_x2 = take(B * W0 * H0 * 128 * 2); p.off_x3 = take(B * W0 * H0 * 256 * 2);
+  p.off_p3 = take(B * W1 * H1 * 256 * 2); p.off_x4 = take(B * W1 * H1 * 256 * 2); p.off_x5 = take(B * W1 * H1 * 512 * 2);
+  p.off_p5 = take(B * T * Hf * 512 * 2); p.off_x6 = take(B * T * Hf * 512 * 2); p.off_x7 = take(B * T * Hf * 512 * 2);
+  p.off_sa = take(B * T * Hf * 16 * 2); p.off_sb = take(B * T * Hf * 32 * 2); p.off_d1 = take(B * 64 * 2);
+  p.off_theta = take(B * 6 * 4); p.off_warp = take(B * T * Hf * 512 * 2); p.off_fc9 = take(B * T * 128 * 2);
+  p.off_xw1 = take(B * T * 1024 * 4); p.off_hf = take(B * T * 128 * 2); p.off_hb = take(B * T * 128 * 2);
+  p.off_l1 = take(B * T * 128 * 2); p.off_xw2 = take(B * T * 1024 * 4); p.off_l2 = take(B * T * 256 * 2);
+  p.off_logits = take(B * g.keep() * B2O_MAX_CLASSES * 4);   // sized for the largest alphabet: independent of the weights
   p.bytes = off;
   return p;
 }
@@ -423,16 +426,22 @@ extern "C" int b2o_load_crnn(b2o_ctx* ctx, const b2o_tensor* tensors, int n) {
       G.alg_cout = k * k * cout;                 // 400 of the 512 columns are real
     }
   }
-  // dense layers as 1x1 "convolutions" over a (1,1,rows,K) view
+  // dense layers as 1x1 "convolutions" over a (1,1,rows,K) view; their input widths follow the crop geometry:
+  // Flatten of the (T, Hf, 32) localisation features, Reshape to (T, Hf*512) (recognition.py:275, 282)
   struct Dense { const char* name; int k, n, relu; };
-  const Dense dense[] = {{"stn.dense_a", 11200, 64, 1}, {"fc_9", 3584, 128, 1}};
+  const CrnnGeometry& g = ctx->crnn_geom;
+  const Dense dense[] = {{"stn.dense_a", g.steps() * g.feat_h() * 32, 64, 1}, {"fc_9", g.feat_h() * 512, 128, 1}};
   for (const Dense& d : dense) {
     if (!has_stn && std::string(d.name).rfind("stn.", 0) == 0) continue;
     const int64_t wshape[2] = {d.k, d.n};
     const int64_t vshape[1] = {d.n};
     const b2o_tensor* w = need(ctx, m, std::string(d.name) + ".kernel", 2, wshape);
     const b2o_tensor* b = need(ctx, m, std::string(d.name) + ".bias", 1, vshape);
-    if (!w || !b) return B2O_ERR_WEIGHTS;
+    if (!w || !b) {
+      ctx->set_error(ctx->error + " (expected (" + std::to_string(d.k) + ", " + std::to_string(d.n) + ") for crops of " +
+                     std::to_string(g.height) + " x " + std::to_string(g.width) + ", see b2o_set_crnn_geometry)");
+      return B2O_ERR_WEIGHTS;
+    }
     const float* wd = w->data;
     const int nn = d.n;
     auto wget = [wd, nn](int o, int c, int, int) { return wd[static_cast<size_t>(c) * nn + o]; };
@@ -489,6 +498,21 @@ extern "C" int b2o_load_crnn(b2o_ctx* ctx, const b2o_tensor* tensors, int n) {
     ctx->n_classes = static_cast<int>(K);
   }
   ctx->crnn_loaded = true;
+  return B2O_OK;
+}
+
+extern "C" int b2o_set_crnn_geometry(b2o_ctx* ctx, int height, int width, int rnn_steps_to_discard) {
+  if (!ctx) return B2O_ERR_ARG;
+  if (height < B2O_CRNN_MIN_HEIGHT || height > B2O_CRNN_MAX_HEIGHT || width < B2O_CRNN_MIN_WIDTH || width > B2O_CRNN_MAX_WIDTH ||
+      rnn_steps_to_discard < 0 || rnn_steps_to_discard >= width / 4) {
+    ctx->set_error("b2o_set_crnn_geometry: unsupported geometry " + std::to_string(height) + " x " + std::to_string(width) +
+                   ", " + std::to_string(rnn_steps_to_discard) + " steps discarded");
+    return B2O_ERR_ARG;
+  }
+  if (ctx->crnn_loaded) { ctx->set_error("b2o_set_crnn_geometry: call it before b2o_load_crnn"); return B2O_ERR_STATE; }
+  ctx->crnn_geom.height = height;
+  ctx->crnn_geom.width = width;
+  ctx->crnn_geom.discard = rnn_steps_to_discard;
   return B2O_OK;
 }
 
@@ -600,7 +624,11 @@ extern "C" int b2o_craft_forward(b2o_ctx* ctx, const uint8_t* img, int n, int h,
 }
 
 // ------------------------------------------------------------------------------------------------
-extern "C" size_t b2o_crnn_workspace_bytes(int b) { return b > 0 ? plan_crnn(b).bytes : 0; }
+extern "C" size_t b2o_crnn_workspace_bytes(int b) { return b > 0 ? plan_crnn(b, CrnnGeometry()).bytes : 0; }
+
+extern "C" size_t b2o_crnn_workspace_bytes_for(const b2o_ctx* ctx, int b) {
+  return ctx && b > 0 ? plan_crnn(b, ctx->crnn_geom).bytes : 0;
+}
 
 extern "C" int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in, int b, int32_t* labels, void* ws, size_t ws_bytes,
                                 void* stream) {
@@ -609,16 +637,18 @@ extern "C" int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in, int b, int32_
   DeviceGuard guard(ctx->device);
   if (b == 0) return B2O_OK;
   if (!crnn_in || !labels || !ws || b < 0) { ctx->set_error("b2o_crnn_forward: bad argument"); return B2O_ERR_ARG; }
-  const CrnnPlan p = plan_crnn(b);
+  const CrnnGeometry& g = ctx->crnn_geom;
+  const CrnnPlan p = plan_crnn(b, g);
   if (ws_bytes < p.bytes) { ctx->set_error("b2o_crnn_forward: workspace too small"); return B2O_ERR_WORKSPACE; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* base = reinterpret_cast<uint8_t*>(ws);
   auto V = [&](size_t off, int nn, int hh, int ww, int c) { return make_view(base + off, nn, hh, ww, c); };
   auto L = [&](const char* name) -> const ConvLayer& { return ctx->crnn[name]; };
-  const TensorView x1 = V(p.off_x1, b, 200, 31, 64), x2 = V(p.off_x2, b, 200, 31, 128), x3 = V(p.off_x3, b, 200, 31, 256);
-  const TensorView p3 = V(p.off_p3, b, 100, 15, 256), x4 = V(p.off_x4, b, 100, 15, 256), x5 = V(p.off_x5, b, 100, 15, 512);
-  const TensorView p5 = V(p.off_p5, b, 50, 7, 512), x6 = V(p.off_x6, b, 50, 7, 512), x7 = V(p.off_x7, b, 50, 7, 512);
-  const TensorView sa = V(p.off_sa, b, 50, 7, 16), sb = V(p.off_sb, b, 50, 7, 32);
+  const int W0 = g.width, H0 = g.height, W1 = W0 / 2, H1 = H0 / 2, T = g.steps(), Hf = g.feat_h();
+  const TensorView x1 = V(p.off_x1, b, W0, H0, 64), x2 = V(p.off_x2, b, W0, H0, 128), x3 = V(p.off_x3, b, W0, H0, 256);
+  const TensorView p3 = V(p.off_p3, b, W1, H1, 256), x4 = V(p.off_x4, b, W1, H1, 256), x5 = V(p.off_x5, b, W1, H1, 512);
+  const TensorView p5 = V(p.off_p5, b, T, Hf, 512), x6 = V(p.off_x6, b, T, Hf, 512), x7 = V(p.off_x7, b, T, Hf, 512);
+  const TensorView sa = V(p.off_sa, b, T, Hf, 16), sb = V(p.off_sb, b, T, Hf, 32);
   // conv stack (recognition.py:217-242)
   B2O_RETURN_IF(stem_crnn_run(ctx, L("conv_1"), reinterpret_cast<const __half*>(crnn_in), b, x1, st));
   B2O_RETURN_IF(conv_run(ctx, L("conv_2"), x1, x2, 0, st));
@@ -633,41 +663,41 @@ extern "C" int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in, int b, int32_
   } else {
   // spatial transformer (263-281)
   if (ctx->conv_engine == B2O_CONV_AUTO && L("stn.conv_a_gemm").block_n != 0) {
-    const TensorView y = V(p.off_warp, b, 50, 7, 512);   // the warp buffer is free until stn_sample
+    const TensorView y = V(p.off_warp, b, T, Hf, 512);   // the warp buffer is free until stn_sample
     B2O_RETURN_IF(conv_run(ctx, L("stn.conv_a_gemm"), x7, y, 0, st));
-    B2O_RETURN_IF(stn_col2im_run(ctx, y.ptr, L("stn.conv_a").t1, b, sa.ptr, st));
+    B2O_RETURN_IF(stn_col2im_run(ctx, y.ptr, L("stn.conv_a").t1, b, T, Hf, sa.ptr, st));
   } else {
     B2O_RETURN_IF(conv_run(ctx, L("stn.conv_a"), x7, sa, 0, st));
   }
   B2O_RETURN_IF(conv_run(ctx, L("stn.conv_b"), sa, sb, 0, st));
-  const TensorView sb_flat = make_view(base + p.off_sb, 1, 1, b, 11200), d1 = make_view(base + p.off_d1, 1, 1, b, 64);
+  const TensorView sb_flat = make_view(base + p.off_sb, 1, 1, b, T * Hf * 32), d1 = make_view(base + p.off_d1, 1, 1, b, 64);
   B2O_RETURN_IF(conv_run(ctx, L("stn.dense_a"), sb_flat, d1, 0, st));
   float* theta = reinterpret_cast<float*>(base + p.off_theta);
   B2O_RETURN_IF(stn_theta_run(ctx, d1.ptr, b, theta, st));
-  B2O_RETURN_IF(stn_sample_run(ctx, x7.ptr, theta, b, warped, st));
+  B2O_RETURN_IF(stn_sample_run(ctx, x7.ptr, theta, b, T, Hf, warped, st));
   }
   // reshape + fc_9 (282-290)
-  const TensorView seq_in = make_view(warped, 1, 1, b * 50, 3584), fc9 = make_view(base + p.off_fc9, 1, 1, b * 50, 128);
+  const TensorView seq_in = make_view(warped, 1, 1, b * T, Hf * 512), fc9 = make_view(base + p.off_fc9, 1, 1, b * T, 128);
   B2O_RETURN_IF(conv_run(ctx, L("fc_9"), seq_in, fc9, 0, st));
   // BiLSTM (292-319)
-  const TensorView xw1 = make_view(base + p.off_xw1, 1, 1, b * 50, 1024);
+  const TensorView xw1 = make_view(base + p.off_xw1, 1, 1, b * T, 1024);
   TensorView xw1v = xw1;      // fp32 output: the view's pointer arithmetic is done by the engine in floats
   B2O_RETURN_IF(conv_run(ctx, L("lstm_in_1"), fc9, xw1v, 1, st));
   __half* hf = reinterpret_cast<__half*>(base + p.off_hf);
   __half* hb = reinterpret_cast<__half*>(base + p.off_hb);
   __half* l1 = reinterpret_cast<__half*>(base + p.off_l1);
   const float* xw1f = reinterpret_cast<const float*>(base + p.off_xw1);
-  B2O_RETURN_IF(lstm_run(ctx, xw1f, 1024, 0, ctx->lstm_u[0], b, 0, hf, 128, 0, st));
-  B2O_RETURN_IF(lstm_run(ctx, xw1f, 1024, 512, ctx->lstm_u[1], b, 1, hb, 128, 0, st));
-  B2O_RETURN_IF(add_run(ctx, hf, hb, l1, static_cast<long long>(b) * 50 * 128, st));
-  const TensorView l1v = make_view(l1, 1, 1, b * 50, 128), xw2 = make_view(base + p.off_xw2, 1, 1, b * 50, 1024);
+  B2O_RETURN_IF(lstm_run(ctx, xw1f, 1024, 0, ctx->lstm_u[0], b, T, 0, hf, 128, 0, st));
+  B2O_RETURN_IF(lstm_run(ctx, xw1f, 1024, 512, ctx->lstm_u[1], b, T, 1, hb, 128, 0, st));
+  B2O_RETURN_IF(add_run(ctx, hf, hb, l1, static_cast<long long>(b) * T * 128, st));
+  const TensorView l1v = make_view(l1, 1, 1, b * T, 128), xw2 = make_view(base + p.off_xw2, 1, 1, b * T, 1024);
   B2O_RETURN_IF(conv_run(ctx, L("lstm_in_2"), l1v, xw2, 1, st));
   const float* xw2f = reinterpret_cast<const float*>(base + p.off_xw2);
   __half* l2 = reinterpret_cast<__half*>(base + p.off_l2);
-  B2O_RETURN_IF(lstm_run(ctx, xw2f, 1024, 0, ctx->lstm_u[2], b, 0, l2, 256, 0, st));
-  B2O_RETURN_IF(lstm_run(ctx, xw2f, 1024, 512, ctx->lstm_u[3], b, 1, l2, 256, 128, st));
+  B2O_RETURN_IF(lstm_run(ctx, xw2f, 1024, 0, ctx->lstm_u[2], b, T, 0, l2, 256, 0, st));
+  B2O_RETURN_IF(lstm_run(ctx, xw2f, 1024, 512, ctx->lstm_u[3], b, T, 1, l2, 256, 128, st));
   // fc_12 + discard + greedy CTC (321-333)
-  B2O_RETURN_IF(fc_ctc_run(ctx, l2, b, ctx->debug_taps ? reinterpret_cast<float*>(base + p.off_logits) : nullptr, labels, st));
+  B2O_RETURN_IF(fc_ctc_run(ctx, l2, b, T, g.discard, ctx->debug_taps ? reinterpret_cast<float*>(base + p.off_logits) : nullptr, labels, st));
   return B2O_OK;
 }
 
@@ -680,20 +710,21 @@ extern "C" int b2o_set_debug_taps(b2o_ctx* ctx, int on) {
 extern "C" int b2o_crnn_tap(b2o_ctx* ctx, const char* name, const void* ws, int b, void* out, size_t out_bytes, void* stream) {
   if (!ctx || !name || !ws || !out || b <= 0) return B2O_ERR_ARG;
   DeviceGuard guard(ctx->device);
-  const CrnnPlan p = plan_crnn(b);
-  const size_t B = static_cast<size_t>(b);
+  const CrnnGeometry& g = ctx->crnn_geom;
+  const CrnnPlan p = plan_crnn(b, g);
+  const size_t B = static_cast<size_t>(b), T = g.steps(), Hf = g.feat_h();
   size_t off = 0, bytes = 0;
   const std::string s(name);
-  if (s == "features") { off = p.off_x7; bytes = B * 50 * 7 * 512 * 2; }
+  if (s == "features") { off = p.off_x7; bytes = B * T * Hf * 512 * 2; }
   else if ((s == "theta" || s == "warped") && !ctx->crnn_stn) { ctx->set_error("b2o_crnn_tap: this recognizer has no spatial transformer"); return B2O_ERR_STATE; }
   else if (s == "theta") { off = p.off_theta; bytes = B * 6 * 4; }
-  else if (s == "warped") { off = p.off_warp; bytes = B * 50 * 7 * 512 * 2; }
-  else if (s == "fc_9") { off = p.off_fc9; bytes = B * 50 * 128 * 2; }
-  else if (s == "l1") { off = p.off_l1; bytes = B * 50 * 128 * 2; }
-  else if (s == "l2") { off = p.off_l2; bytes = B * 50 * 256 * 2; }
+  else if (s == "warped") { off = p.off_warp; bytes = B * T * Hf * 512 * 2; }
+  else if (s == "fc_9") { off = p.off_fc9; bytes = B * T * 128 * 2; }
+  else if (s == "l1") { off = p.off_l1; bytes = B * T * 128 * 2; }
+  else if (s == "l2") { off = p.off_l2; bytes = B * T * 256 * 2; }
   else if (s == "logits") {
     if (!ctx->debug_taps) { ctx->set_error("b2o_crnn_tap: logits are only kept after b2o_set_debug_taps(ctx, 1)"); return B2O_ERR_STATE; }
-    off = p.off_logits; bytes = B * 48 * ctx->n_classes * 4;
+    off = p.off_logits; bytes = B * g.keep() * ctx->n_classes * 4;
   }
   else { ctx->set_error("b2o_crnn_tap: unknown tap " + s); return B2O_ERR_ARG; }
   if (out_bytes < bytes) { ctx->set_error("b2o_crnn_tap: output too small"); return B2O_ERR_ARG; }

@@ -803,14 +803,20 @@ compact_boxes_kernel(const float* __restrict__ boxes, const int32_t* __restrict_
   for (int t = threadIdx.x; t < c; t += blockDim.x) image_index[off + t] = i;
 }
 
-constexpr int kSteps = 48;                         // label steps per word (recognition.py:20: 50 - 2 discarded)
+constexpr int kDefaultSteps = 48;                  // label steps per word at the default geometry (recognition.py:20: 50 - 2)
 
+// label int8 slots of one word: `steps` bytes, the label area rounded up to whole floats per word
+__host__ __device__ inline size_t label_floats(int steps) { return (static_cast<size_t>(steps) + 3) / 4; }
+
+// steps = label row length (T - rnn_steps_to_discard of the recognizer); the words' labels lie back to back as int8
+// in the record's rec_boxes * ceil(steps / 4) label floats, every byte past the last stored word -1
 __global__ void __launch_bounds__(128)
 pack_records_kernel(const float* __restrict__ boxes, const int32_t* __restrict__ counts,
                     const int32_t* __restrict__ labels, const float* __restrict__ inv_scale, int n, int max_boxes,
-                    int rec_boxes, float* __restrict__ rec) {
+                    int rec_boxes, int steps, float* __restrict__ rec) {
   const int row = blockIdx.x;
-  const int rec_len = 1 + rec_boxes * 8 + rec_boxes * (kSteps / 4);
+  const int lab_bytes = rec_boxes * static_cast<int>(label_floats(steps)) * 4;
+  const int rec_len = 1 + rec_boxes * 8 + lab_bytes / 4;
   float* r = rec + static_cast<size_t>(row) * rec_len;
   int8_t* lab = reinterpret_cast<int8_t*>(r + 1 + rec_boxes * 8);
   int c = 0, off = 0, held = 0;
@@ -827,9 +833,9 @@ pack_records_kernel(const float* __restrict__ boxes, const int32_t* __restrict__
   const float* src = boxes + static_cast<size_t>(min(row, n - 1)) * max_boxes * 8;
   for (int t = threadIdx.x; t < rec_boxes * 8; t += blockDim.x)
     r[1 + t] = t < c * 8 ? __fmul_rn(src[t], inv) : 0.f;                  // tools.adjust_boxes (tools.py:232-260)
-  for (int t = threadIdx.x; t < rec_boxes * kSteps; t += blockDim.x) {
-    const int k = t / kSteps;
-    lab[t] = (k < c && labels) ? static_cast<int8_t>(labels[static_cast<size_t>(off + k) * kSteps + (t - k * kSteps)])
+  for (int t = threadIdx.x; t < lab_bytes; t += blockDim.x) {
+    const int k = t / steps;
+    lab[t] = (k < c && labels) ? static_cast<int8_t>(labels[static_cast<size_t>(off + k) * steps + (t - k * steps)])
                    : static_cast<int8_t>(-1);
   }
 }
@@ -850,21 +856,30 @@ extern "C" int b2o_compact_boxes(b2o_ctx* ctx, const float* boxes, const int32_t
   return B2O_OK;
 }
 
-extern "C" size_t b2o_record_floats(int rec_boxes) {
-  return rec_boxes > 0 ? 1 + static_cast<size_t>(rec_boxes) * 8 + static_cast<size_t>(rec_boxes) * (kSteps / 4) : 0;
+extern "C" size_t b2o_record_floats_steps(int rec_boxes, int steps) {
+  return rec_boxes > 0 && steps > 0 ? 1 + static_cast<size_t>(rec_boxes) * 8 + static_cast<size_t>(rec_boxes) * label_floats(steps) : 0;
+}
+
+extern "C" size_t b2o_record_floats(int rec_boxes) { return b2o_record_floats_steps(rec_boxes, kDefaultSteps); }
+
+extern "C" int b2o_pack_records_steps(b2o_ctx* ctx, const float* boxes, const int32_t* counts, const int32_t* labels,
+                                      const float* inv_scale, int n, int max_boxes, int rows, int rec_boxes, int steps,
+                                      float* records, void* stream) {
+  if (!ctx) return B2O_ERR_ARG;
+  DeviceGuard guard(ctx->device);
+  if (!boxes || !counts || !inv_scale || !records || n <= 0 || rows < n || max_boxes <= 0 || rec_boxes <= 0 || steps <= 0) {
+    ctx->set_error("b2o_pack_records: bad argument");      // labels may be NULL when no image has a box
+    return B2O_ERR_ARG;
+  }
+  pack_records_kernel<<<rows, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(boxes, counts, labels, inv_scale, n,
+                                                                              max_boxes, rec_boxes, steps, records);
+  B2O_LAUNCH_CHECK(ctx);
+  return B2O_OK;
 }
 
 extern "C" int b2o_pack_records(b2o_ctx* ctx, const float* boxes, const int32_t* counts, const int32_t* labels,
                                 const float* inv_scale, int n, int max_boxes, int rows, int rec_boxes, float* records,
                                 void* stream) {
-  if (!ctx) return B2O_ERR_ARG;
-  DeviceGuard guard(ctx->device);
-  if (!boxes || !counts || !inv_scale || !records || n <= 0 || rows < n || max_boxes <= 0 || rec_boxes <= 0) {
-    ctx->set_error("b2o_pack_records: bad argument");      // labels may be NULL when no image has a box
-    return B2O_ERR_ARG;
-  }
-  pack_records_kernel<<<rows, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(boxes, counts, labels, inv_scale, n,
-                                                                              max_boxes, rec_boxes, records);
-  B2O_LAUNCH_CHECK(ctx);
-  return B2O_OK;
+  return b2o_pack_records_steps(ctx, boxes, counts, labels, inv_scale, n, max_boxes, rows, rec_boxes, kDefaultSteps,
+                                records, stream);
 }

@@ -85,6 +85,16 @@ struct TensorView {            // NHWC fp16 activation living inside a (possibly
   int ld = 0;                  // channel stride of the underlying buffer (elements)
 };
 
+// Crop geometry of the CRNN (build_model's height / width / rnn_steps_to_discard, recognition.py:13-23, 214, 328).  The
+// conv stack sees a (width, height) image (Permute((2,1,3))); both 2x2 max pools floor, so the features are (T, Hf) =
+// (width // 4, height // 4) and the LSTMs run T steps, of which the first `discard` are dropped before the CTC decode.
+struct CrnnGeometry {
+  int height = 31, width = 200, discard = 2;
+  int steps() const { return width / 4; }            // T
+  int feat_h() const { return height / 4; }          // Hf
+  int keep() const { return width / 4 - discard; }   // label row length (CTC input_length)
+};
+
 struct b2o_ctx {
   int device = 0;
   int sm_count = 148;
@@ -110,6 +120,7 @@ struct b2o_ctx {
   bool craft_loaded = false, crnn_loaded = false;
   int crnn_in_ch = 1;              // 1 = gray crops (default), 3 = RGB crops (build_model(color=True))
   bool crnn_stn = true;            // the loaded CRNN has a spatial transformer (build_model(stn=True), the default)
+  CrnnGeometry crnn_geom;          // b2o_set_crnn_geometry (default 31 x 200, 2 steps discarded)
   bool quads_configured = false;   // quads_kernel's dynamic shared-memory opt-in done on this device
   // CRNN tail parameters (device)
   float *stn_d2_w = nullptr, *stn_d2_b = nullptr;              // dense 64 -> 6, fp32

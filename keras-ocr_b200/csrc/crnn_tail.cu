@@ -5,7 +5,7 @@
 //   lstm_kernel        keras.layers.LSTM x4 (292-318): gates [i,f,c,o], sigmoid/tanh, go_backwards
 //                      outputs kept in processing order; recurrent matrix column-resident in registers
 //   add_kernel         keras.layers.Add (305)
-//   fc_ctc_kernel      Dense(256->37) (322-327; softmax skipped: argmax-invariant), [:, 2:] (328),
+//   fc_ctc_kernel      Dense(256->37) (322-327; softmax skipped: argmax-invariant), [:, discard:] (328),
 //                      greedy CTC with repeat merge + blank removal, -1 padding (169-184)
 #include <math.h>
 
@@ -29,7 +29,7 @@ __device__ __forceinline__ float linspace_pm1(int i, int n) {
   return (i < n / 2) ? (-1.0f + step * static_cast<float>(i)) : (1.0f - step * static_cast<float>(n - 1 - i));
 }
 
-// feat/out: (B, Hh, Ww, C) fp16 with Hh = 50 ("height" of the STN, the time axis), Ww = 7.
+// feat/out: (B, Hh, Ww, C) fp16 with Hh = T ("height" of the STN, the time axis; 50 at 31 x 200), Ww = Hf (7).
 __global__ void stn_sample_kernel(const __half* __restrict__ feat, const float* __restrict__ theta, int B, int Hh,
                                   int Ww, int C, __half* __restrict__ out) {
   // blockIdx.y walks the crops: the index inside one crop is 32-bit (the 64-bit div/mod chain was most of the kernel)
@@ -78,12 +78,11 @@ __global__ void stn_sample_kernel(const __half* __restrict__ feat, const float* 
 }
 
 // ---------------------------------------------------------------------------------------- STN conv_a tail
-// y: (B,50,7,512) fp16, column tap*16 + c = <x[pixel], W[tap][:, c]>; out[p][c] = relu(bias[c] + sum over the
-// 25 taps of y[p + offset(tap)][tap*16 + c]) with zero padding ("same", recognition.py:268-270).  One thread
-// per output pixel, taps added in (ky, kx) order in fp32.
-__global__ void stn_col2im_kernel(const __half* __restrict__ y, const float* __restrict__ bias, int B,
+// y: (B,H,W,512) fp16 with (H, W) = (T, Hf) of the features, column tap*16 + c = <x[pixel], W[tap][:, c]>;
+// out[p][c] = relu(bias[c] + sum over the 25 taps of y[p + offset(tap)][tap*16 + c]) with zero padding ("same",
+// recognition.py:268-270).  One thread per output pixel, taps added in (ky, kx) order in fp32.
+__global__ void stn_col2im_kernel(const __half* __restrict__ y, const float* __restrict__ bias, int B, int H, int W,
                                   __half* __restrict__ out) {
-  constexpr int H = 50, W = 7;
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= B * H * W) return;
   const int w = p % W, h = (p / W) % H;
@@ -125,7 +124,7 @@ __global__ void stn_col2im_kernel(const __half* __restrict__ y, const float* __r
 }
 
 // ---------------------------------------------------------------------------------------- LSTM
-constexpr int kUnits = 128, kGates = 512, kSteps = 50;
+constexpr int kUnits = 128, kGates = 512;
 constexpr int kCropsPerCta = 8;
 constexpr int kHPitch = kUnits + 8;      // halves per crop row of h: +16 B so the 8 crops hit different banks
 
@@ -137,20 +136,21 @@ __device__ __forceinline__ void mma_m16n8k16(float* d, const uint32_t* a, uint32
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
-// One CTA = 8 crops, 16 warps, 50 strictly sequential steps, so what matters is the latency of one step.  The
-// recurrent product z[512 gates x 8 crops] = U^T[512 x 128] . h^T[128 x 8] is exactly the m16n8k16 warp MMA
+// One CTA = 8 crops, 16 warps, T strictly sequential steps (50 for 31 x 200 crops), so what matters is the latency of
+// one step.  The recurrent product z[512 gates x 8 crops] = U^T[512 x 128] . h^T[128 x 8] is exactly the m16n8k16 warp MMA
 // shape with the crops as N: warp w owns units 8w..8w+7 and keeps its two 16-row slices of U^T
 // ({i,f} gates and {c,o} gates of those units, all 128 k) in registers for the whole sequence; the D fragment
 // then hands every thread all four gates of one unit for two crops, so the gate arithmetic needs no exchange
 // and the only shared data is the fp16 h vector (double-buffered, one __syncthreads per step).  tcgen05 does
 // not apply: M = 128 rows would be 94 % padding and its issue -> commit -> tcgen05.ld round trip is longer
 // than this whole step.  h is rounded to fp16 between steps -- the same value that is written to `out`.
+// T   : time steps (crop width / 4)
 // xw  : (B*T, xw_ld) fp32 input projections x@W + b; this direction's 512 gate columns start at xw_off
 // u   : (128, 512) fp16 recurrent kernel (row k = previous-h unit, column g = gate; Keras order i,f,c,o)
 // out : (B, T, out_ld) fp16, written at channel offset out_off, indexed by PROCESSING step
 __global__ void __launch_bounds__(kGates, 1)
-lstm_kernel(const float* __restrict__ xw, int xw_ld, int xw_off, const __half* __restrict__ u, int B, int backwards,
-            __half* __restrict__ out, int out_ld, int out_off) {
+lstm_kernel(const float* __restrict__ xw, int xw_ld, int xw_off, const __half* __restrict__ u, int B, int T,
+            int backwards, __half* __restrict__ out, int out_ld, int out_off) {
   __shared__ __align__(16) __half h_s[2][kCropsPerCta][kHPitch];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r = lane >> 2, q = lane & 3;
@@ -181,8 +181,8 @@ lstm_kernel(const float* __restrict__ xw, int xw_ld, int xw_off, const __half* _
   // input projections of (crop cA / cA+1) x (gates i,f,c,o of `unit`), prefetched one step ahead
   const bool okA = cA < nb, okB = cA + 1 < nb;
   auto load_x = [&](int t, float* z) {
-    const float* pa = xw + (static_cast<size_t>(b0 + cA) * kSteps + t) * xw_ld + xw_off + unit;
-    const float* pb = pa + static_cast<size_t>(kSteps) * xw_ld;
+    const float* pa = xw + (static_cast<size_t>(b0 + cA) * T + t) * xw_ld + xw_off + unit;
+    const float* pb = pa + static_cast<size_t>(T) * xw_ld;
 #pragma unroll
     for (int gidx = 0; gidx < 4; ++gidx) {
       z[2 * gidx] = okA ? pa[gidx * kUnits] : 0.0f;
@@ -190,14 +190,14 @@ lstm_kernel(const float* __restrict__ xw, int xw_ld, int xw_off, const __half* _
     }
   };
   float xnext[8];
-  load_x(backwards ? kSteps - 1 : 0, xnext);
+  load_x(backwards ? T - 1 : 0, xnext);
   float c_state[2] = {0.0f, 0.0f};
   __syncthreads();
-  for (int step = 0; step < kSteps; ++step) {
+  for (int step = 0; step < T; ++step) {
     // D fragments: d0 = {i[cA], i[cB], f[cA], f[cB]}, d1 = {c[cA], c[cB], o[cA], o[cB]}
     float d0[4] = {xnext[0], xnext[1], xnext[2], xnext[3]};
     float d1[4] = {xnext[4], xnext[5], xnext[6], xnext[7]};
-    if (step + 1 < kSteps) load_x(backwards ? (kSteps - 2 - step) : (step + 1), xnext);
+    if (step + 1 < T) load_x(backwards ? (T - 2 - step) : (step + 1), xnext);
     const __half* hrow = &h_s[step & 1][r][q * 2];     // B fragment: h[crop r][k0 .. k0+1], [k0+8 .. k0+9]
 #pragma unroll
     for (int kt = 0; kt < kUnits / 16; ++kt) {
@@ -213,7 +213,7 @@ lstm_kernel(const float* __restrict__ xw, int xw_ld, int xw_off, const __half* _
       const __half h = __float2half_rn(sigmoidf_acc(zo) * tanhf(c));
       c_state[e] = c;
       h_s[(step + 1) & 1][cA + e][unit] = h;
-      if (cA + e < nb) out[(static_cast<size_t>(b0 + cA + e) * kSteps + step) * out_ld + out_off + unit] = h;
+      if (cA + e < nb) out[(static_cast<size_t>(b0 + cA + e) * T + step) * out_ld + out_off + unit] = h;
     }
     __syncthreads();
   }
@@ -227,68 +227,78 @@ __global__ void add_kernel(const __half2* __restrict__ a, const __half2* __restr
 }
 
 // ---------------------------------------------------------------------------------------- fc_12 + CTC
-constexpr int kKeep = 48, kDiscard = 2, kFeat = 256, kFcWarps = 8, kStepsPerWarp = kKeep / kFcWarps;
+constexpr int kFeat = 256, kFcWarps = 8, kStepsPerWarp = 6, kStepsPerPass = kFcWarps * kStepsPerWarp;
+constexpr int kMaxKeep = B2O_CRNN_MAX_WIDTH / 4;
 
-// One CTA per crop, one warp per 6 kept time steps; lane l owns classes l, l+32, ... (K = len(alphabet)+1 is a
-// run-time value: recognition.py:376-381 sizes the Dense layer from the alphabet).  Every logit is the same
-// serial fmaf chain over the 256 features in ascending order whatever K is; the argmax keeps the first maximum
-// (np.argmax / tf.argmax tie rule) and the collapse drops blanks (index K-1) and repeats.
+// One CTA per crop, one warp per 6 kept time steps of a pass over 48 steps (one pass at the default 48 kept steps);
+// lane l owns classes l, l+32, ... (K = len(alphabet)+1 is a run-time value: recognition.py:376-381 sizes the Dense
+// layer from the alphabet).  Every logit is the same serial fmaf chain over the 256 features in ascending order
+// whatever K and the geometry are; the argmax keeps the first maximum (np.argmax / tf.argmax tie rule).  Each pass
+// leaves its per-step argmax in shared memory, and the collapse over all kept steps drops blanks (index K-1) and
+// repeats once every pass is done.
 __global__ void __launch_bounds__(32 * kFcWarps)
-fc_ctc_kernel(const __half* __restrict__ l2 /*[B][50][256]*/, const float* __restrict__ w /*[256][K]*/,
-              const float* __restrict__ bias, int B, int K, float* __restrict__ logits /*[B][48][K] or null*/,
-              int* __restrict__ labels /*[B][48]*/) {
-  __shared__ int best[kKeep];
-  __shared__ __half xs[kKeep][kFeat];
+fc_ctc_kernel(const __half* __restrict__ l2 /*[B][T][256]*/, const float* __restrict__ w /*[256][K]*/,
+              const float* __restrict__ bias, int B, int K, int T, int discard,
+              float* __restrict__ logits /*[B][T-discard][K] or null*/, int* __restrict__ labels /*[B][T-discard]*/) {
+  __shared__ int best[kMaxKeep];
+  __shared__ __half xs[kStepsPerPass][kFeat];
   const int b = blockIdx.x;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(l2 + (static_cast<size_t>(b) * kSteps + kDiscard) * kFeat);
-    uint4* dst = reinterpret_cast<uint4*>(&xs[0][0]);
-    for (int i = threadIdx.x; i < kKeep * kFeat / 8; i += blockDim.x) dst[i] = src[i];
-  }
-  __syncthreads();
-  const int t0 = warp * kStepsPerWarp;
-  float mx[kStepsPerWarp];
-  int arg[kStepsPerWarp];
+  const int keep = T - discard;
+  for (int pass = 0; pass < keep; pass += kStepsPerPass) {
+    const int rows = min(kStepsPerPass, keep - pass);
+    if (pass > 0) __syncthreads();                     // the previous pass is done with xs
+    {
+      const uint4* src = reinterpret_cast<const uint4*>(l2 + (static_cast<size_t>(b) * T + discard + pass) * kFeat);
+      uint4* dst = reinterpret_cast<uint4*>(&xs[0][0]);
+      for (int i = threadIdx.x; i < rows * kFeat / 8; i += blockDim.x) dst[i] = src[i];
+    }
+    __syncthreads();
+    const int t0 = warp * kStepsPerWarp;
+    if (t0 < rows) {                                   // warp-uniform
+      float mx[kStepsPerWarp];
+      int arg[kStepsPerWarp];
 #pragma unroll
-  for (int j = 0; j < kStepsPerWarp; ++j) { mx[j] = -INFINITY; arg[j] = 0x7fffffff; }
-  for (int k = lane; k < K; k += 32) {
-    float acc[kStepsPerWarp];
-    const float bk = bias[k];
+      for (int j = 0; j < kStepsPerWarp; ++j) { mx[j] = -INFINITY; arg[j] = 0x7fffffff; }
+      for (int k = lane; k < K; k += 32) {
+        float acc[kStepsPerWarp];
+        const float bk = bias[k];
 #pragma unroll
-    for (int j = 0; j < kStepsPerWarp; ++j) acc[j] = bk;
+        for (int j = 0; j < kStepsPerWarp; ++j) acc[j] = bk;
 #pragma unroll 4
-    for (int c = 0; c < kFeat; ++c) {
-      const float wv = __ldg(w + static_cast<size_t>(c) * K + k);
+        for (int c = 0; c < kFeat; ++c) {
+          const float wv = __ldg(w + static_cast<size_t>(c) * K + k);
 #pragma unroll
-      for (int j = 0; j < kStepsPerWarp; ++j) acc[j] = fmaf(__half2float(xs[t0 + j][c]), wv, acc[j]);
+          for (int j = 0; j < kStepsPerWarp; ++j) acc[j] = fmaf(__half2float(xs[t0 + j][c]), wv, acc[j]);
+        }
+#pragma unroll
+        for (int j = 0; j < kStepsPerWarp; ++j) {
+          if (acc[j] > mx[j]) { mx[j] = acc[j]; arg[j] = k; }            // ascending k: first maximum wins
+          if (logits && t0 + j < rows) logits[(static_cast<size_t>(b) * keep + pass + t0 + j) * K + k] = acc[j];
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < kStepsPerWarp; ++j) {
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+          const float om = __shfl_xor_sync(0xffffffffu, mx[j], off);
+          const int oa = __shfl_xor_sync(0xffffffffu, arg[j], off);
+          if (om > mx[j] || (om == mx[j] && oa < arg[j])) { mx[j] = om; arg[j] = oa; }
+        }
+        if (lane == 0 && t0 + j < rows) best[pass + t0 + j] = arg[j] == 0x7fffffff ? 0 : arg[j];  // all-NaN row: argmax returns 0
+      }
     }
-#pragma unroll
-    for (int j = 0; j < kStepsPerWarp; ++j) {
-      if (acc[j] > mx[j]) { mx[j] = acc[j]; arg[j] = k; }            // ascending k: first maximum wins
-      if (logits) logits[(static_cast<size_t>(b) * kKeep + t0 + j) * K + k] = acc[j];
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < kStepsPerWarp; ++j) {
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-      const float om = __shfl_xor_sync(0xffffffffu, mx[j], off);
-      const int oa = __shfl_xor_sync(0xffffffffu, arg[j], off);
-      if (om > mx[j] || (om == mx[j] && oa < arg[j])) { mx[j] = om; arg[j] = oa; }
-    }
-    if (lane == 0) best[t0 + j] = arg[j] == 0x7fffffff ? 0 : arg[j];  // all-NaN row: argmax returns 0
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    int* o = labels + static_cast<size_t>(b) * kKeep;
+    int* o = labels + static_cast<size_t>(b) * keep;
     int n = 0, prev = -1;
-    for (int s = 0; s < kKeep; ++s) {
+    for (int s = 0; s < keep; ++s) {
       const int c = best[s];
       if (c != K - 1 && c != prev) o[n++] = c;
       prev = c;
     }
-    for (; n < kKeep; ++n) o[n] = -1;
+    for (; n < keep; ++n) o[n] = -1;
   }
 }
 
@@ -302,23 +312,23 @@ int stn_theta_run(b2o_ctx* ctx, const __half* d1, int B, float* theta, cudaStrea
   return B2O_OK;
 }
 
-int stn_col2im_run(b2o_ctx* ctx, const __half* y, const float* bias, int B, __half* out, cudaStream_t st) {
-  const int total = B * 50 * 7;
-  stn_col2im_kernel<<<(total + 127) / 128, 128, 0, st>>>(y, bias, B, out);
+int stn_col2im_run(b2o_ctx* ctx, const __half* y, const float* bias, int B, int H, int W, __half* out, cudaStream_t st) {
+  const int total = B * H * W;
+  stn_col2im_kernel<<<(total + 127) / 128, 128, 0, st>>>(y, bias, B, H, W, out);
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
 }
 
-int stn_sample_run(b2o_ctx* ctx, const __half* feat, const float* theta, int B, __half* out, cudaStream_t st) {
+int stn_sample_run(b2o_ctx* ctx, const __half* feat, const float* theta, int B, int Hh, int Ww, __half* out, cudaStream_t st) {
   if (B <= 0) return B2O_OK;
-  stn_sample_kernel<<<dim3(nb(50 * 7 * (512 / 8), 256), B < 65535 ? B : 65535), 256, 0, st>>>(feat, theta, B, 50, 7, 512, out);
+  stn_sample_kernel<<<dim3(nb(Hh * Ww * (512 / 8), 256), B < 65535 ? B : 65535), 256, 0, st>>>(feat, theta, B, Hh, Ww, 512, out);
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
 }
 
-int lstm_run(b2o_ctx* ctx, const float* xw, int xw_ld, int xw_off, const __half* u, int B, int backwards, __half* out,
+int lstm_run(b2o_ctx* ctx, const float* xw, int xw_ld, int xw_off, const __half* u, int B, int T, int backwards, __half* out,
              int out_ld, int out_off, cudaStream_t st) {
-  lstm_kernel<<<(B + kCropsPerCta - 1) / kCropsPerCta, kGates, 0, st>>>(xw, xw_ld, xw_off, u, B, backwards, out, out_ld,
+  lstm_kernel<<<(B + kCropsPerCta - 1) / kCropsPerCta, kGates, 0, st>>>(xw, xw_ld, xw_off, u, B, T, backwards, out, out_ld,
                                                                         out_off);
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
@@ -331,8 +341,9 @@ int add_run(b2o_ctx* ctx, const __half* a, const __half* b, __half* o, long long
   return B2O_OK;
 }
 
-int fc_ctc_run(b2o_ctx* ctx, const __half* l2, int B, float* logits, int* labels, cudaStream_t st) {
-  fc_ctc_kernel<<<B, 32 * kFcWarps, 0, st>>>(l2, ctx->fc12_w, ctx->fc12_b, B, ctx->n_classes, logits, labels);
+int fc_ctc_run(b2o_ctx* ctx, const __half* l2, int B, int T, int discard, float* logits, int* labels, cudaStream_t st) {
+  if (T - discard < 1 || T - discard > kMaxKeep) { ctx->set_error("fc_ctc_run: unsupported step count"); return B2O_ERR_ARG; }
+  fc_ctc_kernel<<<B, 32 * kFcWarps, 0, st>>>(l2, ctx->fc12_w, ctx->fc12_b, B, ctx->n_classes, T, discard, logits, labels);
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
 }

@@ -174,29 +174,29 @@ __device__ void plan_warp(const float* q /*4x2*/, int target_w, int target_h, Wa
   plan->valid = 1;
 }
 
-constexpr int kCropH = 31, kCropW = 200;
-
-// CH = 1: gray image (n,H,W), crops (k,31,200), CRNN input (k,200,31).  CH = 3 (build_model(color=True),
-// recognition.py:214, 508-510: no gray conversion): RGB image (n,H,W,3), crops (k,31,200,3), CRNN input (k,200,31,3);
-// cv2.warpPerspective samples every channel with the same coordinates and weights.
+// CH = 1: gray image (n,H,W), crops (k,ch,cw), CRNN input (k,cw,ch).  CH = 3 (build_model(color=True),
+// recognition.py:214, 508-510: no gray conversion): RGB image (n,H,W,3), crops (k,ch,cw,3), CRNN input (k,cw,ch,3);
+// cv2.warpPerspective samples every channel with the same coordinates and weights.  (ch, cw) = the recognizer's crop
+// size (31 x 200 by default); the crop is staged in dynamic shared memory (ch * cw * CH bytes).
 template <int CH>
 __global__ void __launch_bounds__(256)
 warp_kernel(const uint8_t* __restrict__ gray, int n, int H, int W, const float* __restrict__ boxes,
-            const int* __restrict__ image_index, uint8_t* __restrict__ crops, __half* __restrict__ crnn_in) {
+            const int* __restrict__ image_index, int crop_h, int crop_w, uint8_t* __restrict__ crops,
+            __half* __restrict__ crnn_in) {
   __shared__ WarpPlan plan;
-  __shared__ uint8_t tile[kCropH * kCropW * CH];
+  extern __shared__ uint8_t tile[];
   const int k = blockIdx.x;
-  if (threadIdx.x == 0) plan_warp(boxes + static_cast<size_t>(k) * 8, kCropW, kCropH, &plan);
+  if (threadIdx.x == 0) plan_warp(boxes + static_cast<size_t>(k) * 8, crop_w, crop_h, &plan);
   __syncthreads();
   int img = image_index[k];
   img = min(max(img, 0), n - 1);
   const uint8_t* g = gray + static_cast<size_t>(img) * H * W * CH;
-  const int dw = plan.valid ? min(plan.dw, kCropW) : 0, dh = plan.valid ? min(plan.dh, kCropH) : 0;
+  const int dw = plan.valid ? min(plan.dw, crop_w) : 0, dh = plan.valid ? min(plan.dh, crop_h) : 0;
   // block structure of cv::WarpPerspectiveInvoker (decides where X0/Y0/W0 are re-based)
   int bh0 = min(16, max(dh, 1));
   const int bw0 = min(1024 / bh0, max(dw, 1));
-  for (int i = threadIdx.x; i < kCropH * kCropW; i += blockDim.x) {
-    const int y = i / kCropW, x = i - y * kCropW;
+  for (int i = threadIdx.x; i < crop_h * crop_w; i += blockDim.x) {
+    const int y = i / crop_w, x = i - y * crop_w;
     int v[CH];
 #pragma unroll
     for (int c = 0; c < CH; ++c) v[c] = 0;
@@ -230,30 +230,32 @@ warp_kernel(const uint8_t* __restrict__ gray, int n, int H, int W, const float* 
 #pragma unroll
     for (int c = 0; c < CH; ++c) {
       tile[i * CH + c] = static_cast<uint8_t>(v[c]);
-      if (crops) crops[(static_cast<size_t>(k) * kCropH * kCropW + i) * CH + c] = static_cast<uint8_t>(v[c]);
+      if (crops) crops[(static_cast<size_t>(k) * crop_h * crop_w + i) * CH + c] = static_cast<uint8_t>(v[c]);
     }
   }
   if (crnn_in == nullptr) return;
   __syncthreads();
-  // CRNN input layout (recognition.py:215-216): x[t][j] = crop[30-j][t] / 255
-  __half* o = crnn_in + static_cast<size_t>(k) * kCropH * kCropW * CH;
-  for (int i = threadIdx.x; i < kCropH * kCropW * CH; i += blockDim.x) {
+  // CRNN input layout (recognition.py:215-216): x[t][j] = crop[ch-1-j][t] / 255
+  __half* o = crnn_in + static_cast<size_t>(k) * crop_h * crop_w * CH;
+  for (int i = threadIdx.x; i < crop_h * crop_w * CH; i += blockDim.x) {
     const int c = i % CH, q = i / CH;
-    const int t = q / kCropH, j = q - t * kCropH;
-    o[i] = __float2half_rn(static_cast<float>(tile[((kCropH - 1 - j) * kCropW + t) * CH + c]) / 255.0f);
+    const int t = q / crop_h, j = q - t * crop_h;
+    o[i] = __float2half_rn(static_cast<float>(tile[((crop_h - 1 - j) * crop_w + t) * CH + c]) / 255.0f);
   }
 }
 
-// crops (k,31,200[,ch]) u8 -> CRNN input (k,200,31[,ch]) fp16 = crop / 255 after Permute((2,1,3)) and the axis flip
-__global__ void crops_to_input_kernel(const uint8_t* __restrict__ crops, long long total, int ch, __half* __restrict__ out) {
+// crops (k,crop_h,crop_w[,ch]) u8 -> CRNN input (k,crop_w,crop_h[,ch]) fp16 = crop / 255 after Permute((2,1,3)) and the
+// axis flip
+__global__ void crops_to_input_kernel(const uint8_t* __restrict__ crops, long long total, int ch, int crop_h, int crop_w,
+                                      __half* __restrict__ out) {
   const long long p = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (p >= total) return;
-  const int per = kCropH * kCropW * ch;
+  const int per = crop_h * crop_w * ch;
   const long long k = p / per;
   const int i = static_cast<int>(p - k * per);
   const int c = i % ch, q = i / ch;
-  const int t = q / kCropH, j = q - t * kCropH;
-  out[p] = __float2half_rn(static_cast<float>(crops[k * per + ((kCropH - 1 - j) * kCropW + t) * ch + c]) / 255.0f);
+  const int t = q / crop_h, j = q - t * crop_h;
+  out[p] = __float2half_rn(static_cast<float>(crops[k * per + ((crop_h - 1 - j) * crop_w + t) * ch + c]) / 255.0f);
 }
 
 }  // namespace
@@ -309,8 +311,16 @@ static int warp_boxes_impl(b2o_ctx* ctx, const uint8_t* img, int ch, int n, int 
     return B2O_ERR_ARG;
   }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (ch == 3) warp_kernel<3><<<n_boxes, 256, 0, st>>>(img, n, h, w, boxes, image_index, crops, reinterpret_cast<__half*>(crnn_in));
-  else warp_kernel<1><<<n_boxes, 256, 0, st>>>(img, n, h, w, boxes, image_index, crops, reinterpret_cast<__half*>(crnn_in));
+  const int chh = ctx->crnn_geom.height, cw = ctx->crnn_geom.width;
+  const size_t smem = static_cast<size_t>(chh) * cw * ch;
+  const void* fn = ch == 3 ? reinterpret_cast<const void*>(warp_kernel<3>) : reinterpret_cast<const void*>(warp_kernel<1>);
+  if (smem > 48 * 1024 && !ctx->configured.count(fn)) {      // crops past 48 KB (e.g. 64 x 800 RGB): opt in once per device
+    B2O_CUDA_CHECK(ctx, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             static_cast<int>(static_cast<size_t>(B2O_CRNN_MAX_HEIGHT) * B2O_CRNN_MAX_WIDTH * 3)));
+    ctx->configured.insert(fn);
+  }
+  if (ch == 3) warp_kernel<3><<<n_boxes, 256, smem, st>>>(img, n, h, w, boxes, image_index, chh, cw, crops, reinterpret_cast<__half*>(crnn_in));
+  else warp_kernel<1><<<n_boxes, 256, smem, st>>>(img, n, h, w, boxes, image_index, chh, cw, crops, reinterpret_cast<__half*>(crnn_in));
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
 }
@@ -330,9 +340,10 @@ static int crops_to_input_impl(b2o_ctx* ctx, const uint8_t* crops, int ch, int b
   DeviceGuard guard(ctx->device);
   if (b == 0) return B2O_OK;
   if (!crops || !crnn_in || b < 0) { ctx->set_error("b2o_crops_to_input: bad argument"); return B2O_ERR_ARG; }
-  const long long total = static_cast<long long>(b) * kCropH * kCropW * ch;
+  const int chh = ctx->crnn_geom.height, cw = ctx->crnn_geom.width;
+  const long long total = static_cast<long long>(b) * chh * cw * ch;
   crops_to_input_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      crops, total, ch, reinterpret_cast<__half*>(crnn_in));
+      crops, total, ch, chh, cw, reinterpret_cast<__half*>(crnn_in));
   B2O_LAUNCH_CHECK(ctx);
   return B2O_OK;
 }

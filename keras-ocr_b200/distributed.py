@@ -3,14 +3,24 @@
 The reference is single-process (SURVEY.md 2.3); images are fully independent in
 ``Pipeline.recognize`` (reference pipeline.py:28-75), so the path shards with no data-path
 collective.  Each rank runs the whole pipeline on its contiguous slice and the per-image result
-records -- ``count`` (int32), ``boxes`` (M,4,2) float32, ``labels`` (M,48) int8 -- are gathered to
-rank 0 with a single ``torch.distributed.gather`` over NCCL/NVLink (``gloo`` in the CPU tests).
+records -- ``count`` (int32), ``boxes`` (M,4,2) float32, ``labels`` (M,steps) int8 -- are gathered to
+rank 0 with a single ``torch.distributed.gather`` over NCCL/NVLink (``gloo`` in the CPU tests).  ``steps`` is the
+recognizer's label row length (``Recognizer.steps``: 48 for the default 31 x 200 crops).
 """
 import numpy as np
 import torch
 import torch.distributed as dist
 
-STEPS = 48
+STEPS = 48                                             # label row length of the default recognizer
+
+
+def label_slots(steps):
+    """float32 slots per word of a record's label area: ``steps`` int8 labels, 4 per slot (b2o_record_floats_steps)."""
+    return (int(steps) + 3) // 4
+
+
+def _steps_of(pipeline):
+    return int(getattr(pipeline.recognizer, "steps", STEPS))
 
 
 def shard_bounds(n_items, world_size, rank):
@@ -20,15 +30,18 @@ def shard_bounds(n_items, world_size, rank):
     return lo, lo + base + (1 if rank < extra else 0)
 
 
-def pack_records(counts, boxes, labels, per_rank, max_boxes):
-    """Fixed-size record block for one rank: float32 tensor (per_rank, 1 + max_boxes*8 + max_boxes*12).
+def pack_records(counts, boxes, labels, per_rank, max_boxes, steps=STEPS):
+    """Fixed-size record block for one rank: float32 tensor (per_rank, 1 + max_boxes*8 + max_boxes*ceil(steps/4)).
 
-    labels (int8, 48 per word) are bit-packed 4 per float32 slot so that a single dtype travels.
-    counts (n,), boxes (n,M,4,2) float32, labels (sum(counts),48) int -> one contiguous CPU tensor.
+    labels (int8, ``steps`` per word) are bit-packed 4 per float32 slot so that a single dtype travels; the words'
+    labels lie back to back and the bytes after the last one are -1 (the layout of b2o_pack_records_steps).
+    counts (n,), boxes (n,M,4,2) float32, labels (sum(counts),steps) int -> one contiguous CPU tensor.
     """
     n = len(counts)
-    rec = np.zeros((per_rank, 1 + max_boxes * 8 + max_boxes * (STEPS // 4)), dtype=np.float32)
-    lab8 = np.full((per_rank, max_boxes, STEPS), -1, dtype=np.int8)
+    slots = label_slots(steps)
+    rec = np.zeros((per_rank, 1 + max_boxes * 8 + max_boxes * slots), dtype=np.float32)
+    lab_area = np.full((per_rank, max_boxes * slots * 4), -1, dtype=np.int8)
+    lab8 = lab_area[:, :max_boxes * steps].reshape(per_rank, max_boxes, steps)
     start = 0
     for i in range(n):
         c = min(int(counts[i]), max_boxes)
@@ -37,14 +50,14 @@ def pack_records(counts, boxes, labels, per_rank, max_boxes):
         if c:
             lab8[i, :c] = np.asarray(labels[start:start + c], dtype=np.int8)
         start += int(counts[i])
-    rec[:, 1 + max_boxes * 8:] = lab8.reshape(per_rank, -1).view(np.float32)
+    rec[:, 1 + max_boxes * 8:] = lab_area.view(np.float32)
     rec[n:, 0] = -1                                    # padding rows of a short last shard
     return torch.from_numpy(rec)
 
 
-def unpack_records(rec, max_boxes):
-    """Inverse of pack_records for one rank's block -> list of (count, boxes (c,4,2), labels (c,48))."""
-    counts, boxes, labels = unpack_blocks([rec], max_boxes)
+def unpack_records(rec, max_boxes, steps=STEPS):
+    """Inverse of pack_records for one rank's block -> list of (count, boxes (c,4,2), labels (c,steps))."""
+    counts, boxes, labels = unpack_blocks([rec], max_boxes, steps=steps)
     ends = np.cumsum(counts)
     return [(int(c), boxes[e - c:e], labels[e - c:e].astype(np.int32)) for c, e in zip(counts, ends)]
 
@@ -53,9 +66,9 @@ class RecordOverflow(ValueError):
     """An image has more words than a fixed-size record holds (``max_boxes``)."""
 
 
-def unpack_blocks(blocks, max_boxes, strict=True):
+def unpack_blocks(blocks, max_boxes, strict=True, steps=STEPS):
     """All gathered blocks at once (rank order = global image order): returns (counts (n_images,), boxes (total,4,2)
-    float32, labels (total,48) int8) with the words of image i at [sum(counts[:i]), +counts[i]).  Only the used
+    float32, labels (total,steps) int8) with the words of image i at [sum(counts[:i]), +counts[i]).  Only the used
     prefix of every record is touched (two concatenations of per-image views), not the 75 % padding.
 
     A record's count field is the number of words its image HAS; a record holds ``max_boxes`` of them.  The
@@ -78,9 +91,9 @@ def unpack_blocks(blocks, max_boxes, strict=True):
             counts.append(c)
             if c:
                 box_parts.append(rec[i, 1:1 + c * 8])
-                lab_parts.append(rec8[i, lab0:lab0 + c * STEPS])
+                lab_parts.append(rec8[i, lab0:lab0 + c * steps])
     boxes = np.concatenate(box_parts).reshape(-1, 4, 2) if box_parts else np.zeros((0, 4, 2), np.float32)
-    labels = np.concatenate(lab_parts).reshape(-1, STEPS) if lab_parts else np.zeros((0, STEPS), np.int8)
+    labels = np.concatenate(lab_parts).reshape(-1, steps) if lab_parts else np.zeros((0, steps), np.int8)
     return np.asarray(counts, dtype=np.int64), boxes, labels
 
 
@@ -95,21 +108,21 @@ def gather_records(local, world_size, rank, device=None):
     return blocks
 
 
-def _host_records(pipeline, local, per_rank, max_boxes):
+def _host_records(pipeline, local, per_rank, max_boxes, steps=STEPS):
     """Record block of a duck-typed pipeline: pack the (word, box) lists its ``recognize`` returned on the host."""
     alphabet = pipeline.recognizer.alphabet
     counts = [len(g) for g in local]
     boxes = [np.array([b for _, b in g], dtype=np.float32).reshape(-1, 4, 2) for g in local]
-    labels = np.full((sum(counts), STEPS), -1, dtype=np.int8)
+    labels = np.full((sum(counts), steps), -1, dtype=np.int8)
     k = 0
     for g in local:
         for text, _ in g:
             labels[k, :len(text)] = [alphabet.index(ch) for ch in text]
             k += 1
-    return pack_records(counts, boxes, labels, per_rank, max_boxes)
+    return pack_records(counts, boxes, labels, per_rank, max_boxes, steps)
 
 
-def recognize_sharded(pipeline, images, max_boxes=128, presharded=False):
+def recognize_sharded(pipeline, images, max_boxes=128, presharded=False, steps=None):
     """Run ``pipeline.recognize`` on this rank's shard of ``images`` and gather to rank 0.
 
     ``images`` is the global batch (every rank passes the same list and takes its contiguous slice) or, with
@@ -119,9 +132,12 @@ def recognize_sharded(pipeline, images, max_boxes=128, presharded=False):
     NCCL/NVLink, and copied to the host once, on rank 0.  Any other pipeline goes through ``recognize`` and
     ``pack_records``.
 
+    ``steps``: label row length of the records (default: ``pipeline.recognizer.steps``, 48 for the default recognizer).
+
     Returns, on rank 0, the same list-of-lists as ``Pipeline.recognize`` for ALL images (global
     order); ``None`` on the other ranks.  Boxes are in source-image pixels.
     """
+    steps = _steps_of(pipeline) if steps is None else int(steps)
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
     if presharded:
@@ -148,12 +164,12 @@ def recognize_sharded(pipeline, images, max_boxes=128, presharded=False):
         result = pipeline.recognize(mine) if len(mine) else []
         if max_boxes == "auto":
             max_boxes = agree_max_boxes([len(g) for g in result], _collective_device(pipeline))
-        local = _host_records(pipeline, result, per_rank, max_boxes)
+        local = _host_records(pipeline, result, per_rank, max_boxes, steps)
         device = _collective_device(pipeline)
     blocks = gather_records(local, world, rank, device)
     if rank != 0:
         return None
-    return _decode_blocks(blocks, max_boxes, alphabet)
+    return _decode_blocks(blocks, max_boxes, alphabet, steps)
 
 
 def _collective_device(pipeline):
@@ -180,21 +196,21 @@ def agree_max_boxes(counts, device=None, floor=16):
 stats = {"decode_ms": 0.0, "decodes": 0}      # rank 0's serial host work (bench.py reports it per step)
 
 
-def _decode_blocks(blocks, max_boxes, alphabet):
+def _decode_blocks(blocks, max_boxes, alphabet, steps=STEPS):
     import time
 
     from . import recognition
 
     t0 = time.perf_counter()
     try:
-        return _decode_blocks_impl(blocks, max_boxes, alphabet, recognition)
+        return _decode_blocks_impl(blocks, max_boxes, alphabet, recognition, steps)
     finally:
         stats["decode_ms"] += (time.perf_counter() - t0) * 1e3
         stats["decodes"] += 1
 
 
-def _decode_blocks_impl(blocks, max_boxes, alphabet, recognition):
-    counts, boxes, labels = unpack_blocks(blocks, max_boxes)
+def _decode_blocks_impl(blocks, max_boxes, alphabet, recognition, steps):
+    counts, boxes, labels = unpack_blocks(blocks, max_boxes, steps=steps)
     texts = recognition.labels_to_text(labels, alphabet)
     quads, out, start = list(boxes), [], 0             # one (4,2) view per word, made once
     for c in counts.tolist():
@@ -216,10 +232,12 @@ class ShardedStream:
     With this package's ``Pipeline`` the records stay on the device until the gather and reach the host through ONE
     asynchronous copy into pinned memory; any other pipeline (``recognize`` only) is served too, without the overlap.
     ``max_boxes``: words a record holds (an image with more raises ``RecordOverflow`` on rank 0 when its batch is
-    decoded) or ``"auto"`` (sized per batch by ``agree_max_boxes``)."""
+    decoded) or ``"auto"`` (sized per batch by ``agree_max_boxes``).  ``steps``: label row length of the records
+    (default: ``pipeline.recognizer.steps``, 48 for the default recognizer)."""
 
-    def __init__(self, pipeline, max_boxes=128):
+    def __init__(self, pipeline, max_boxes=128, steps=None):
         self.pipeline, self.max_boxes = pipeline, max_boxes
+        self.steps = _steps_of(pipeline) if steps is None else int(steps)
         self.world = dist.get_world_size() if dist.is_initialized() else 1
         self.rank = dist.get_rank() if dist.is_initialized() else 0
         self.alphabet = pipeline.recognizer.alphabet
@@ -238,7 +256,7 @@ class ShardedStream:
         self._pending = None
         if event is not None:
             event.synchronize()
-        return _decode_blocks(list(host), max_boxes, self.alphabet)
+        return _decode_blocks(list(host), max_boxes, self.alphabet, self.steps)
 
     def submit(self, images):
         rows = len(images)
@@ -257,7 +275,7 @@ class ShardedStream:
             result = self.pipeline.recognize(images)
             if max_boxes == "auto":
                 max_boxes = agree_max_boxes([len(g) for g in result], _collective_device(self.pipeline))
-            local = _host_records(self.pipeline, result, rows, max_boxes)
+            local = _host_records(self.pipeline, result, rows, max_boxes, self.steps)
             device = _collective_device(self.pipeline)
         if local.is_cuda or device is not None:
             self._gather_on_side_stream(local.to(device) if device is not None else local, max_boxes)

@@ -198,9 +198,9 @@ class Pipeline:
 
     def recognize_records(self, images, rows=None, rec_boxes=128, detection_kwargs=None):
         """``recognize`` without the trip to the host: returns the results as a CUDA float32 tensor of fixed-size
-        per-image records, ``(rows, b2o_record_floats(rec_boxes))`` = [count | rec_boxes x (4,2) boxes in source
-        pixels | rec_boxes x 48 int8 labels] (``distributed.unpack_blocks`` decodes it; rows beyond ``len(images)``
-        carry count -1).  This is the payload of the multi-GPU gather (SURVEY.md 8(e)): only the per-image box
+        per-image records, ``(rows, b2o_record_floats_steps(rec_boxes, steps))`` = [count | rec_boxes x (4,2) boxes in
+        source pixels | rec_boxes x steps int8 labels], steps = ``recognizer.steps`` (48 for the default recognizer;
+        ``distributed.unpack_blocks(..., steps=steps)`` decodes it; rows beyond ``len(images)`` carry count -1).  This is the payload of the multi-GPU gather (SURVEY.md 8(e)): only the per-image box
         counts ever reach the host on this rank."""
         return self.records_end(self.records_begin(images, rows, rec_boxes, detection_kwargs))
 
@@ -246,7 +246,7 @@ class Pipeline:
         det, rec = self.detector, self.recognizer
         n, rows = state["n"], state["rows"]
         rec_boxes = state["rec_boxes"] if rec_boxes is None else int(rec_boxes)
-        records = torch.empty((rows, det.ctx.record_floats(rec_boxes)), dtype=torch.float32, device=det.device)
+        records = torch.empty((rows, det.ctx.record_floats(rec_boxes, rec.steps)), dtype=torch.float32, device=det.device)
         if n == 0:
             records.zero_()
             records[:, 0] = -1
@@ -260,7 +260,7 @@ class Pipeline:
         inv = torch.tensor([1.0 / s for s in st["scales"]], dtype=torch.float32).to(det.device, non_blocking=True)
         det.ctx.pack_records(boxes.data_ptr(), bst["counts"].data_ptr(), labels.data_ptr() if labels is not None else None,
                              inv.data_ptr(), n, boxes.shape[1], rows, rec_boxes, records.data_ptr(),
-                             torch.cuda.current_stream(det.device).cuda_stream)
+                             torch.cuda.current_stream(det.device).cuda_stream, steps=rec.steps)
         self.last_stats["d2h_bytes"] = int(counts.nbytes)
         return records
 

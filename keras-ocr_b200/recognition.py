@@ -8,7 +8,8 @@ import torch
 from . import _lib, tools, weights as weights_mod
 
 DEFAULT_ALPHABET = string.digits + string.ascii_lowercase      # reference recognition.py:25
-TARGET_HEIGHT, TARGET_WIDTH, STEPS = 31, 200, 48                # DEFAULT_BUILD_PARAMS, recognition.py:13-23
+TARGET_HEIGHT, TARGET_WIDTH, STEPS = 31, 200, 48                # DEFAULT_BUILD_PARAMS, recognition.py:13-23 (the defaults;
+                                                                # a Recognizer's own are its height / width / steps)
 DEFAULT_BUILD_PARAMS = {"height": 31, "width": 200, "color": False, "filters": (64, 128, 256, 256, 512, 512, 512),
                         "rnn_units": (128, 128), "dropout": 0.25, "rnn_steps_to_discard": 2, "pool_size": 2}
 
@@ -46,22 +47,32 @@ class Recognizer:
             (read with h5py where installed) in the cache dir; otherwise a ``.npz`` / ``.h5`` path or a dict
             keyed like ``weights.py``.
         build_params: ``None`` / the defaults (reference recognition.py:13-23), optionally with ``"stn": False`` (the
-            recognizer without the spatial transformer, recognition.py:243) and / or ``"color": True`` (RGB crops into a
-            3-channel ``conv_1``, recognition.py:214); other architectures raise NotImplementedError.
+            recognizer without the spatial transformer, recognition.py:243), ``"color": True`` (RGB crops into a
+            3-channel ``conv_1``, recognition.py:214), another crop size ``"height"`` / ``"width"`` and another
+            ``"rnn_steps_to_discard"`` (recognition.py:214, 328); ``"dropout"`` is accepted and has no effect at
+            inference.  Crops are ``height x width``; the model reads ``T = width // 4`` time steps and returns label
+            rows of ``T - rnn_steps_to_discard`` (the instance's ``steps``; 48 by default).  Supported: height 16..64,
+            width 32..800, ``0 <= rnn_steps_to_discard < width // 4`` -- ValueError otherwise.  Other ``filters``,
+            ``rnn_units`` or ``pool_size`` raise NotImplementedError.
     """
 
     def __init__(self, alphabet=None, weights="kurapan", build_params=None, device=None):
         assert alphabet or weights, "At least one of alphabet or weights must be provided."
-        # build_params (recognition.py:13-23, 365-368): the CUDA recognizer implements the default architecture; of the
-        # build options only ``stn`` (with / without the spatial transformer, recognition.py:243) and ``color`` (RGB instead
-        # of gray crops, recognition.py:214) may differ
+        # build_params (recognition.py:13-23, 365-368): the CUDA recognizer implements the default layer stack; of the
+        # build options ``stn`` (with / without the spatial transformer, recognition.py:243), ``color`` (RGB instead of
+        # gray crops, recognition.py:214), the crop size and the discarded steps (214, 328) may differ, and ``dropout``
+        # is an inference no-op (321)
         params = dict(DEFAULT_BUILD_PARAMS, **(build_params or {}))
         self.stn = bool(params.pop("stn", True))
-        self.color = bool(params["color"])                        # RGB crops, no gray conversion (recognition.py:214, 508-510)
-        params["color"] = False
-        if params != DEFAULT_BUILD_PARAMS:
-            changed = sorted(k for k in params if params[k] != DEFAULT_BUILD_PARAMS.get(k))
+        self.color = bool(params.pop("color"))                    # RGB crops, no gray conversion (recognition.py:214, 508-510)
+        self.height, self.width = params.pop("height"), params.pop("width")
+        self.rnn_steps_to_discard = params.pop("rnn_steps_to_discard")
+        params.pop("dropout")
+        changed = sorted(k for k in params if params[k] != DEFAULT_BUILD_PARAMS.get(k))
+        if changed:
             raise NotImplementedError(f"build_params other than the defaults are not supported by the CUDA recognizer: {changed}")
+        self._check_geometry()
+        self.steps = self.width // 4 - self.rnn_steps_to_discard  # label row length (CTC input_length)
         if not torch.cuda.is_available():
             raise _lib.B2OError("keras-ocr_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.alphabet = alphabet or DEFAULT_ALPHABET              # recognition.py:369-375
@@ -74,7 +85,8 @@ class Recognizer:
             tensors = weights
         elif weights is None:
             # reference recognition.py:382-383: no weights -> the freshly built (untrained) model for this alphabet
-            tensors = weights_mod.synthetic_crnn_weights(seed=0, alphabet=self.alphabet, stn=self.stn, color=self.color)
+            tensors = weights_mod.synthetic_crnn_weights(seed=0, alphabet=self.alphabet, stn=self.stn, color=self.color,
+                                                         height=self.height, width=self.width)
         elif isinstance(weights, str) and weights.endswith(".npz"):
             tensors = weights_mod.load_npz(weights)
         elif isinstance(weights, str) and weights.endswith(".h5"):
@@ -94,6 +106,7 @@ class Recognizer:
             tensors = {k: v for k, v in tensors.items() if not k.startswith("stn.")}
         elif self.stn and not has_stn:
             raise ValueError("the checkpoint has no spatial-transformer tensors: pass build_params={'stn': False}")
+        self._check_checkpoint_geometry(tensors)
         in_ch = int(np.shape(tensors["conv_1.kernel"])[2]) if "conv_1.kernel" in tensors else 1
         if in_ch != (3 if self.color else 1):
             raise ValueError(f"conv_1.kernel takes {in_ch} input channel(s): pass build_params={{'color': {in_ch == 3}}}")
@@ -106,10 +119,42 @@ class Recognizer:
             tensors["fc_12.kernel"] = np.random.default_rng(0).uniform(-limit, limit, (256, n_classes)).astype(np.float32)
             tensors["fc_12.bias"] = np.zeros(n_classes, np.float32)
         self.ctx = _lib.Context(self.device_index)
+        self.ctx.set_crnn_geometry(self.height, self.width, self.rnn_steps_to_discard)
         self.ctx.load_crnn(tensors)
         self._keep_workspace = False     # tests set keep_workspace to read intermediate taps
         self._last_ws = None
         self._ws = None                  # reusable CRNN workspace (grown on demand)
+
+    def _check_geometry(self):
+        """The crop size and discarded steps the kernels support (include/b2ocr.h, b2o_set_crnn_geometry)."""
+        (h_lo, h_hi), (w_lo, w_hi) = _lib.CRNN_HEIGHTS, _lib.CRNN_WIDTHS
+        for key, value in (("height", self.height), ("width", self.width), ("rnn_steps_to_discard", self.rnn_steps_to_discard)):
+            if isinstance(value, bool) or not isinstance(value, (int, np.integer)):
+                raise ValueError(f"build_params[{key!r}] must be an integer, got {value!r}")
+        self.height, self.width, self.rnn_steps_to_discard = int(self.height), int(self.width), int(self.rnn_steps_to_discard)
+        if not h_lo <= self.height <= h_hi or not w_lo <= self.width <= w_hi:
+            raise ValueError(f"crops of {self.height} x {self.width} are not supported: height {h_lo}..{h_hi}, width {w_lo}..{w_hi}")
+        if not 0 <= self.rnn_steps_to_discard < self.width // 4:
+            raise ValueError(f"rnn_steps_to_discard={self.rnn_steps_to_discard} must be in 0..{self.width // 4 - 1}: "
+                             f"crops {self.width} wide give {self.width // 4} time steps")
+
+    def _check_checkpoint_geometry(self, tensors):
+        """fc_9 reads height // 4 * 512 features per step and stn.dense_a the flattened (width // 4, height // 4, 32)
+        localisation map (recognition.py:275, 282): a checkpoint built for another crop size does not fit."""
+        feat_h, t = self.height // 4, self.width // 4
+        fc9 = tensors.get("fc_9.kernel")
+        if fc9 is not None and int(np.shape(fc9)[0]) != feat_h * 512:
+            rows = int(np.shape(fc9)[0])
+            hint = (f"pass build_params with a 'height' in {4 * (rows // 512)}..{4 * (rows // 512) + 3}" if rows % 512 == 0
+                    else "no crop height fits it")
+            raise ValueError(f"fc_9.kernel has {rows} rows but crops {self.height} high need {feat_h * 512}: {hint}")
+        dense = tensors.get("stn.dense_a.kernel") if self.stn else None
+        if dense is not None and int(np.shape(dense)[0]) != t * feat_h * 32:
+            rows = int(np.shape(dense)[0])
+            hint = (f"pass build_params with a 'width' in {4 * (rows // (feat_h * 32))}..{4 * (rows // (feat_h * 32)) + 3}"
+                    if rows % (feat_h * 32) == 0 else "no crop width fits it")
+            raise ValueError(f"stn.dense_a.kernel has {rows} rows but {self.height} x {self.width} crops need "
+                             f"{t * feat_h * 32}: {hint}")
 
     @property
     def keep_workspace(self):
@@ -131,23 +176,24 @@ class Recognizer:
 
     def warp_device(self, gray, boxes_flat, image_index, want_crops=False):
         """tools.warpBox for every box.  ``gray``: (N,H,W) u8 -- or the RGB batch (N,H,W,3) for a color recognizer.
-        Returns (crnn_in (B,200,31[,3]) fp16, crops (B,31,200[,3]) u8 or None)."""
+        Returns (crnn_in (B,width,height[,3]) fp16, crops (B,height,width[,3]) u8 or None); 200 x 31 by default."""
         n, h, w = gray.shape[:3]
         color = gray.dim() == 4
         assert color == self.color, "a color recognizer warps the RGB batch, a gray one the gray batch"
         tail = (3,) if color else ()
         b = boxes_flat.shape[0]
-        crnn_in = torch.empty((b, TARGET_WIDTH, TARGET_HEIGHT) + tail, dtype=torch.float16, device=self.device)
-        crops = torch.empty((b, TARGET_HEIGHT, TARGET_WIDTH) + tail, dtype=torch.uint8, device=self.device) if want_crops else None
+        crnn_in = torch.empty((b, self.width, self.height) + tail, dtype=torch.float16, device=self.device)
+        crops = torch.empty((b, self.height, self.width) + tail, dtype=torch.uint8, device=self.device) if want_crops else None
         self.ctx.warp_boxes(gray.data_ptr(), n, h, w, boxes_flat.data_ptr(), image_index.data_ptr(), b,
                             crops.data_ptr() if want_crops else None, crnn_in.data_ptr(),
                             torch.cuda.current_stream(self.device).cuda_stream, color=color)
         return crnn_in, crops
 
     def predict_device(self, crnn_in):
-        """CRNN + greedy CTC.  crnn_in: (B,200,31) fp16 -> labels (B,48) int32 (-1 padded)."""
+        """CRNN + greedy CTC.  crnn_in: (B,width,height) fp16 -> labels (B,steps) int32 (-1 padded); (B,200,31) -> (B,48)
+        by default."""
         b = crnn_in.shape[0]
-        labels = torch.empty((b, STEPS), dtype=torch.int32, device=self.device)
+        labels = torch.empty((b, self.steps), dtype=torch.int32, device=self.device)
         nbytes = self.ctx.crnn_workspace_bytes(b)
         if self._ws is None or self._ws.numel() < nbytes:
             self._ws = None
@@ -167,30 +213,32 @@ class Recognizer:
         return out
 
     def recognize_crops(self, crops):
-        """crops: (B,31,200) uint8 -- (B,31,200,3) for a color recognizer -- i.e. what tools.warpBox returns -> list[str]."""
+        """crops: (B,height,width) uint8 -- (B,height,width,3) for a color recognizer -- i.e. what tools.warpBox returns at
+        the model's crop size (31 x 200 by default) -> list[str]."""
         t = crops if isinstance(crops, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(crops))
         t = t.to(self.device).contiguous()
         b = t.shape[0]
         if b == 0:
             return []
-        assert t.shape[1:] == (TARGET_HEIGHT, TARGET_WIDTH) + ((3,) if self.color else ()), "crops must be (B,31,200[,3])"
-        crnn_in = torch.empty((b, TARGET_WIDTH, TARGET_HEIGHT) + ((3,) if self.color else ()), dtype=torch.float16, device=self.device)
+        tail = (3,) if self.color else ()
+        assert t.shape[1:] == (self.height, self.width) + tail, f"crops must be (B,{self.height},{self.width}{',3' if tail else ''})"
+        crnn_in = torch.empty((b, self.width, self.height) + tail, dtype=torch.float16, device=self.device)
         self.ctx.crops_to_input(t.data_ptr(), b, crnn_in.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream,
                                 color=self.color)
         return labels_to_text(self.predict_device(crnn_in).cpu().numpy(), self.alphabet)
 
     def recognize(self, image):
-        """Recognize text from a single pre-cropped image (reference recognition.py:467-489): fit to
-        200x31 with zero fill (host, as upstream), gray conversion, then the CUDA CRNN."""
+        """Recognize text from a single pre-cropped image (reference recognition.py:467-489): fit to the model's
+        width x height (200 x 31 by default) with zero fill (host, as upstream), gray conversion, then the CUDA CRNN."""
         import cv2
 
-        image = tools.read_and_fit(filepath_or_array=image, width=TARGET_WIDTH, height=TARGET_HEIGHT, cval=0)
+        image = tools.read_and_fit(filepath_or_array=image, width=self.width, height=self.height, cval=0)
         if not self.color and image.ndim == 3 and image.shape[-1] == 3:      # recognition.py:481-483
             image = cv2.cvtColor(image, code=cv2.COLOR_RGB2GRAY)
-        return self.recognize_crops(np.ascontiguousarray(image.reshape((1, TARGET_HEIGHT, TARGET_WIDTH) + ((3,) if self.color else ()))))[0]
+        return self.recognize_crops(np.ascontiguousarray(image.reshape((1, self.height, self.width) + ((3,) if self.color else ()))))[0]
 
     def recognize_from_boxes_device(self, images_t, boxes, counts, gray=None, flat=None, image_index=None):
-        """images_t (N,H,W,3) u8 CUDA; boxes (N,M,4,2) f32 CUDA; counts host ndarray -> labels (B,48) i32 CUDA.
+        """images_t (N,H,W,3) u8 CUDA; boxes (N,M,4,2) f32 CUDA; counts host ndarray -> labels (B,steps) i32 CUDA.
 
         Optional device-side by-products of the earlier stages, so that nothing but the kernel launches is
         left to do once the host knows the counts: ``gray`` (N,H,W) u8 from ``b2o_resize_pad_batch``;

@@ -146,11 +146,13 @@ def synthetic_craft_weights(seed=0, textlike=False):
 HERSHEY = "crnn_hershey.npz"                # keras-ocr_b200/data/: the reference CRNN trained on rendered words (see below)
 
 
-def synthetic_crnn_weights(seed=1, alphabet=ALPHABET, decisive=False, stn=True, color=False):
+def synthetic_crnn_weights(seed=1, alphabet=ALPHABET, decisive=False, stn=True, color=False, height=31, width=200):
     """Seeded CRNN weights keyed by Keras layer name (Keras layouts); the top layer has len(alphabet)+1 classes.
 
     ``color=True``: ``conv_1`` takes 3 input channels (``build_model(color=True)``, recognition.py:214).
     ``stn=False``: no spatial-transformer tensors (the ``build_model(stn=False)`` variant, recognition.py:196, 243).
+    ``height`` / ``width``: the crop size of ``build_model(height, width)``; it sets the input widths of ``fc_9``
+    (``height // 4 * 512``) and ``stn.dense_a`` (``width // 4 * height // 4 * 32``).  The defaults give 31 x 200.
     ``decisive=True`` (default alphabet, gray, with STN; ``seed`` is ignored): every tensor comes from
     ``data/crnn_hershey.npz`` -- the reference architecture TRAINED with CTC loss on words rendered in cv2's Hershey font
     and cut out as the oracle pipeline cuts them (``oracle/train_crnn_full.py``; 3.5 minutes on one B200; no pretrained file
@@ -159,11 +161,13 @@ def synthetic_crnn_weights(seed=1, alphabet=ALPHABET, decisive=False, stn=True, 
     strings can be compared for identity (BASELINE.json north_star) instead of up to the near-ties random weights leave."""
     if decisive:
         import os
-        assert alphabet == ALPHABET and stn and not color, "the trained recognizer is the default architecture / alphabet"
+        assert alphabet == ALPHABET and stn and not color and (height, width) == (31, 200), \
+            "the trained recognizer is the default architecture / alphabet"
         path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", HERSHEY)
         with np.load(path) as data:
             return {k: data[k].astype(np.float32) for k in data.files}
     rng = np.random.default_rng(seed)
+    steps, feat_h = width // 4, height // 4          # both 2x2 max pools floor (recognition.py:227, 235)
     w = {}
     for name, cin, cout, k, bn in CRNN_CONVS:
         w[name + ".kernel"] = _he(rng, (k, k, cin, cout), cin * k * k)
@@ -177,12 +181,12 @@ def synthetic_crnn_weights(seed=1, alphabet=ALPHABET, decisive=False, stn=True, 
     w["stn.conv_a.bias"] = (rng.standard_normal(16) * 0.05).astype(np.float32)
     w["stn.conv_b.kernel"] = _he(rng, (5, 5, 16, 32), 16 * 25)
     w["stn.conv_b.bias"] = (rng.standard_normal(32) * 0.05).astype(np.float32)
-    w["stn.dense_a.kernel"] = _he(rng, (11200, 64), 11200)
+    w["stn.dense_a.kernel"] = _he(rng, (steps * feat_h * 32, 64), steps * feat_h * 32)
     w["stn.dense_a.bias"] = (rng.standard_normal(64) * 0.05).astype(np.float32)
     # a trained STN sits near the identity transform [[1,0,0],[0,1,0]] with small deviations
     w["stn.dense_b.kernel"] = (rng.standard_normal((64, 6)) * 0.01).astype(np.float32)
     w["stn.dense_b.bias"] = (np.array([1, 0, 0, 0, 1, 0]) + rng.standard_normal(6) * 0.02).astype(np.float32)
-    w["fc_9.kernel"] = _he(rng, (3584, 128), 3584)
+    w["fc_9.kernel"] = _he(rng, (feat_h * 512, 128), feat_h * 512)
     w["fc_9.bias"] = (rng.standard_normal(128) * 0.05).astype(np.float32)
     for name in CRNN_LSTMS:
         w[name + ".kernel"] = _he(rng, (128, 512), 128, 1.0)
@@ -233,7 +237,8 @@ def map_keras_datasets(flat):
     ``flat`` maps a dataset path such as ``conv_3/conv_3/kernel:0`` or ``lstm_10/lstm_10/lstm_cell/bias:0`` to its
     array.  Named layers of ``build_model`` (reference recognition.py:214-329) map by name; the nested localisation
     model of the spatial transformer is auto-named by Keras (``model_N/conv2d_M/...``, recognition.py:263-277), so its
-    eight tensors are told apart by their shapes, which are all distinct."""
+    eight tensors are told apart by their shapes, which are all distinct (``dense_a``'s kernel by its 64 columns: its
+    row count depends on the crop size)."""
     out = {}
     for path, arr in flat.items():
         parts = [q for q in path.split("/") if q]
@@ -245,6 +250,8 @@ def map_keras_datasets(flat):
             key = f"{parts[0]}.{kind}"
         else:
             key = _STN_BY_SHAPE.get(tuple(arr.shape))
+            if key is None and kind == "kernel" and arr.ndim == 2 and arr.shape[1] == 64:
+                key = "stn.dense_a.kernel"          # Flatten of the (T, Hf, 32) map: rows follow the crop size (build_model height / width)
             if key is None or not key.endswith(kind):
                 raise ValueError(f"unrecognised tensor {path} with shape {arr.shape} in Keras weight file")
         if key in out:
