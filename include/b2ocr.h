@@ -166,6 +166,16 @@ int b2o_crops_to_input(b2o_ctx* ctx, const uint8_t* crops_dev, int b, void* crnn
 /* crops (b,height,width,3) uint8 -> (b,width,height,3) fp16 for a color=True recognizer (conv_1.kernel of shape
  * (3,3,3,64)); b2o_crnn_forward then takes that 3-channel input.                                              */
 int b2o_crops_to_input_color(b2o_ctx* ctx, const uint8_t* crops_dev, int b, void* crnn_in_dev, void* stream);
+/* Recognizer.recognize's preparation (recognition.py:467-489: tools.fit(cval=0) to the context's crop size, then
+ * cv2.cvtColor for a gray model) for b RGB crops of any size at once.  srcs_dev: device array of b device pointers,
+ * crop k being (sh,sw,3) uint8, contiguous; crops may live in one staging buffer or in separate allocations.
+ * dims_dev: b x (sh, sw, rh, rw) int32, where (rh, rw) is the resize size tools.fit picks (tools.fit_plan), and
+ * (rh, rw) = (sh, sw) when it does not resize; a row with a non-positive entry gives an all-zero crop.  crnn_in:
+ * (b,width,height) fp16 -- (b,width,height,3) when the loaded CRNN takes RGB crops -- in the layout of
+ * b2o_crops_to_input; crops_dev (nullable): the fitted RGB crops (b,height,width,3) uint8, what tools.fit returns.
+ * b == 0 is a no-op.                                                                                           */
+int b2o_fit_crops(b2o_ctx* ctx, const uint8_t* const* srcs_dev, const int32_t* dims_dev, int b,
+                  uint8_t* crops_dev, void* crnn_in_dev, void* stream);
 int b2o_crnn_forward(b2o_ctx* ctx, const void* crnn_in_dev, int b, int32_t* labels_dev,
                      void* ws_dev, size_t ws_bytes, void* stream);
 

@@ -60,6 +60,7 @@ SIGNATURES = {
     "b2o_warp_boxes": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "b2o_warp_boxes_color": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "b2o_crops_to_input_color": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "b2o_fit_crops": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "b2o_crnn_workspace_bytes": (_sz, [_i]),
     "b2o_crnn_workspace_bytes_for": (_sz, [_vp, _i]),
     "b2o_crops_to_input": (_i, [_vp, _vp, _i, _vp, _vp]),
@@ -227,6 +228,10 @@ class Context:
     def crops_to_input(self, crops, b, crnn_in, stream, color=False):
         fn = self.lib.b2o_crops_to_input_color if color else self.lib.b2o_crops_to_input
         self._check(fn(self.handle, crops, b, crnn_in, stream), "b2o_crops_to_input")
+
+    def fit_crops(self, srcs, dims, b, crops, crnn_in, stream):
+        """srcs: device array of b crop pointers; dims: device (b, 4) int32 (sh, sw, rh, rw); crops nullable."""
+        self._check(self.lib.b2o_fit_crops(self.handle, srcs, dims, b, crops, crnn_in, stream), "b2o_fit_crops")
 
     def crnn_forward(self, crnn_in, b, labels, ws, ws_bytes, stream):
         self._check(self.lib.b2o_crnn_forward(self.handle, crnn_in, b, labels, ws, ws_bytes, stream), "b2o_crnn_forward")

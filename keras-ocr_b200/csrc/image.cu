@@ -3,6 +3,7 @@
 // tests/test_cv_models.py):
 //   resize_pad_kernel : cv2.resize INTER_LINEAR on uint8 (tools.py:394-396) + tools.pad(255) (356-375)
 //   gray_kernel       : cv2.cvtColor(RGB2GRAY) (recognition.py:510)
+//   fit_crops_kernel  : tools.fit(cval=0) (tools.py:402-452) + cvtColor of ragged crops for Recognizer.recognize
 //   warp_kernel       : tools.warpBox (tools.py:61-117): get_rotated_box ordering (533-581, rectangle
 //                       branch), get_rotated_width_height (41-57), cv2.getPerspectiveTransform (8x8 LU,
 //                       fp64), cv2.warpPerspective INTER_LINEAR (1/32-pixel coordinates, 15-bit weights)
@@ -18,6 +19,34 @@ namespace {
 // recognizer a second pass over the batch.
 __device__ __forceinline__ uint8_t gray_of(int r, int g, int b) {
   return static_cast<uint8_t>((9798 * r + 19235 * g + 3735 * b + 16384) >> 15);
+}
+
+// cv2.resize INTER_LINEAR on uint8 at output pixel (x, y) of an RGB source (hs, ws): OpenCV's scale = 1 / (dsize /
+// ssize), source coordinate at pixel centres, float fractions, 11-bit coefficients (INTER_RESIZE_COEF_BITS),
+// horizontal pass first.  One row or one column is fine: the clamps keep every read inside the source.
+__device__ __forceinline__ void resize_sample(const uint8_t* __restrict__ src, int hs, int ws, int x, int y,
+                                              double scale_x, double scale_y, int rgb[3]) {
+  float fx = static_cast<float>((x + 0.5) * scale_x - 0.5);
+  int sx = static_cast<int>(floorf(fx));
+  fx -= sx;
+  if (sx < 0) { fx = 0.f; sx = 0; }
+  if (sx >= ws - 1) { fx = 0.f; sx = ws - 1; }
+  const int sx1 = min(sx + 1, ws - 1);
+  const int a0 = __float2int_rn((1.f - fx) * 2048.f), a1 = __float2int_rn(fx * 2048.f);
+  float fy = static_cast<float>((y + 0.5) * scale_y - 0.5);
+  const int sy = static_cast<int>(floorf(fy));
+  fy -= sy;
+  const int b0 = __float2int_rn((1.f - fy) * 2048.f), b1 = __float2int_rn(fy * 2048.f);
+  const int y0 = min(max(sy, 0), hs - 1), y1 = min(max(sy + 1, 0), hs - 1);
+  const uint8_t* r0 = src + static_cast<size_t>(y0) * ws * 3;
+  const uint8_t* r1 = src + static_cast<size_t>(y1) * ws * 3;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const int s0 = r0[sx * 3 + c] * a0 + r0[sx1 * 3 + c] * a1;
+    const int s1 = r1[sx * 3 + c] * a0 + r1[sx1 * 3 + c] * a1;
+    const int v = (((b0 * (s0 >> 4)) >> 16) + ((b1 * (s1 >> 4)) >> 16) + 2) >> 2;
+    rgb[c] = min(max(v, 0), 255);
+  }
 }
 
 // scale_x / scale_y = 1 / (dsize / ssize) in fp64, computed once on the host exactly as OpenCV does: two fp64
@@ -36,31 +65,10 @@ __global__ void resize_pad_kernel(const uint8_t* __restrict__ src, int hs, int w
     if (gray) gray[opix] = gray_of(255, 255, 255);
     return;
   }
-  // OpenCV: scale = 1 / (dsize / ssize), source coordinate at pixel centres, float fractions,
-  // 11-bit coefficients (INTER_RESIZE_COEF_BITS), horizontal pass first.
-  float fx = static_cast<float>((x + 0.5) * scale_x - 0.5);
-  int sx = static_cast<int>(floorf(fx));
-  fx -= sx;
-  if (sx < 0) { fx = 0.f; sx = 0; }
-  if (sx >= ws - 1) { fx = 0.f; sx = ws - 1; }
-  const int sx1 = min(sx + 1, ws - 1);
-  const int a0 = __float2int_rn((1.f - fx) * 2048.f), a1 = __float2int_rn(fx * 2048.f);
-  float fy = static_cast<float>((y + 0.5) * scale_y - 0.5);
-  const int sy = static_cast<int>(floorf(fy));
-  fy -= sy;
-  const int b0 = __float2int_rn((1.f - fy) * 2048.f), b1 = __float2int_rn(fy * 2048.f);
-  const int y0 = min(max(sy, 0), hs - 1), y1 = min(max(sy + 1, 0), hs - 1);
-  const uint8_t* r0 = src + static_cast<size_t>(y0) * ws * 3;
-  const uint8_t* r1 = src + static_cast<size_t>(y1) * ws * 3;
   int rgb[3];
+  resize_sample(src, hs, ws, x, y, scale_x, scale_y, rgb);
 #pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    const int s0 = r0[sx * 3 + c] * a0 + r0[sx1 * 3 + c] * a1;
-    const int s1 = r1[sx * 3 + c] * a0 + r1[sx1 * 3 + c] * a1;
-    const int v = (((b0 * (s0 >> 4)) >> 16) + ((b1 * (s1 >> 4)) >> 16) + 2) >> 2;
-    rgb[c] = min(max(v, 0), 255);
-    o[c] = static_cast<uint8_t>(rgb[c]);
-  }
+  for (int c = 0; c < 3; ++c) o[c] = static_cast<uint8_t>(rgb[c]);
   if (gray) gray[opix] = gray_of(rgb[0], rgb[1], rgb[2]);
 }
 
@@ -244,6 +252,13 @@ warp_kernel(const uint8_t* __restrict__ gray, int n, int H, int W, const float* 
   }
 }
 
+// CRNN input layout (recognition.py:215-216, Permute((2,1,3)) and the axis flip): pixel q = t * crop_h + j of a crop's
+// (crop_w, crop_h) input plane reads crop pixel (y, x) = (crop_h - 1 - j, t).
+__device__ __forceinline__ int crnn_in_source_pixel(int q, int crop_h, int crop_w) {
+  const int t = q / crop_h, j = q - t * crop_h;
+  return (crop_h - 1 - j) * crop_w + t;
+}
+
 // crops (k,crop_h,crop_w[,ch]) u8 -> CRNN input (k,crop_w,crop_h[,ch]) fp16 = crop / 255 after Permute((2,1,3)) and the
 // axis flip
 __global__ void crops_to_input_kernel(const uint8_t* __restrict__ crops, long long total, int ch, int crop_h, int crop_w,
@@ -253,9 +268,58 @@ __global__ void crops_to_input_kernel(const uint8_t* __restrict__ crops, long lo
   const int per = crop_h * crop_w * ch;
   const long long k = p / per;
   const int i = static_cast<int>(p - k * per);
-  const int c = i % ch, q = i / ch;
-  const int t = q / crop_h, j = q - t * crop_h;
-  out[p] = __float2half_rn(static_cast<float>(crops[k * per + ((crop_h - 1 - j) * crop_w + t) * ch + c]) / 255.0f);
+  const int c = i % ch;
+  out[p] = __float2half_rn(static_cast<float>(crops[k * per + crnn_in_source_pixel(i / ch, crop_h, crop_w) * ch + c]) / 255.0f);
+}
+
+// ------------------------------------------------------------------------------------ tools.fit of ragged crops
+// Recognizer.recognize's host preparation (recognition.py:467-489: tools.read_and_fit(cval=0), tools.py:402-452, then
+// cvtColor for a gray model) for b RGB crops of any size, one block per crop.  dims[k] = (sh, sw, rh, rw): the
+// source size and the cv2.resize dsize tools.fit picks (tools.fit_plan; rh == sh and rw == sw when fit does not
+// resize).  Pixels inside rh x rw are resize_pad_kernel's sample, the rest of the crop_h x crop_w crop is 0.  Writes
+// the CRNN input (b,crop_w,crop_h[,CH]) in crnn_in_source_pixel order -- CH = 1: gray_of the fitted pixel, CH = 3: RGB
+// -- and, when given, the fitted RGB crops (b,crop_h,crop_w,3), i.e. what tools.fit returns.
+template <int CH>
+__global__ void __launch_bounds__(256)
+fit_crops_kernel(const uint8_t* const* __restrict__ srcs, const int32_t* __restrict__ dims, int crop_h, int crop_w,
+                 uint8_t* __restrict__ crops, __half* __restrict__ crnn_in) {
+  __shared__ double scale[2];
+  const int k = blockIdx.x;
+  const int sh = dims[4 * k], sw = dims[4 * k + 1], rh = dims[4 * k + 2], rw = dims[4 * k + 3];
+  const bool valid = sh > 0 && sw > 0 && rh > 0 && rw > 0;
+  const bool copy = rh == sh && rw == sw;            // cv2.resize copies when dsize == ssize
+  if (threadIdx.x == 0 && valid) {                   // once per crop: fp64 divisions are slow (see resize_pad_kernel)
+    scale[0] = 1.0 / (static_cast<double>(rw) / sw);
+    scale[1] = 1.0 / (static_cast<double>(rh) / sh);
+  }
+  __syncthreads();
+  const uint8_t* src = srcs[k];
+  const int vh = valid ? min(rh, crop_h) : 0, vw = valid ? min(rw, crop_w) : 0;
+  const size_t base = static_cast<size_t>(k) * crop_h * crop_w;
+  for (int q = threadIdx.x; q < crop_h * crop_w; q += blockDim.x) {
+    const int pix = crnn_in_source_pixel(q, crop_h, crop_w);
+    const int y = pix / crop_w, x = pix - y * crop_w;
+    int rgb[3] = {0, 0, 0};
+    if (y < vh && x < vw) {
+      if (copy) {
+        const uint8_t* s = src + (static_cast<size_t>(y) * sw + x) * 3;
+        rgb[0] = s[0]; rgb[1] = s[1]; rgb[2] = s[2];
+      } else {
+        resize_sample(src, sh, sw, x, y, scale[0], scale[1], rgb);
+      }
+    }
+    if (crops) {
+      uint8_t* o = crops + (base + pix) * 3;
+      o[0] = static_cast<uint8_t>(rgb[0]); o[1] = static_cast<uint8_t>(rgb[1]); o[2] = static_cast<uint8_t>(rgb[2]);
+    }
+    __half* o = crnn_in + (base + q) * CH;
+    if (CH == 1) {
+      o[0] = __float2half_rn(static_cast<float>(gray_of(rgb[0], rgb[1], rgb[2])) / 255.0f);
+    } else {
+#pragma unroll
+      for (int c = 0; c < CH; ++c) o[c] = __float2half_rn(static_cast<float>(rgb[c]) / 255.0f);
+    }
+  }
 }
 
 }  // namespace
@@ -354,4 +418,22 @@ extern "C" int b2o_crops_to_input(b2o_ctx* ctx, const uint8_t* crops, int b, voi
 
 extern "C" int b2o_crops_to_input_color(b2o_ctx* ctx, const uint8_t* crops, int b, void* crnn_in, void* stream) {
   return crops_to_input_impl(ctx, crops, 3, b, crnn_in, stream);
+}
+
+extern "C" int b2o_fit_crops(b2o_ctx* ctx, const uint8_t* const* srcs_dev, const int32_t* dims_dev, int b,
+                             uint8_t* crops_dev, void* crnn_in_dev, void* stream) {
+  if (!ctx) return B2O_ERR_ARG;
+  DeviceGuard guard(ctx->device);
+  if (b == 0) return B2O_OK;
+  if (!srcs_dev || !dims_dev || !crnn_in_dev || b < 0) {
+    ctx->set_error("b2o_fit_crops: bad argument (srcs, dims and crnn_in are required, b >= 0)");
+    return B2O_ERR_ARG;
+  }
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int chh = ctx->crnn_geom.height, cw = ctx->crnn_geom.width;
+  __half* out = reinterpret_cast<__half*>(crnn_in_dev);
+  if (ctx->crnn_in_ch == 3) fit_crops_kernel<3><<<b, 256, 0, st>>>(srcs_dev, dims_dev, chh, cw, crops_dev, out);
+  else fit_crops_kernel<1><<<b, 256, 0, st>>>(srcs_dev, dims_dev, chh, cw, crops_dev, out);
+  B2O_LAUNCH_CHECK(ctx);
+  return B2O_OK;
 }

@@ -189,6 +189,39 @@ class Recognizer:
                             torch.cuda.current_stream(self.device).cuda_stream, color=color)
         return crnn_in, crops
 
+    def _fit_dims(self, shape):
+        """(sh, sw, rh, rw) of one (H,W,3) crop for b2o_fit_crops; raises what tools.fit raises for it."""
+        if len(shape) != 3 or shape[2] != 3:
+            raise ValueError(f"crops must be (H, W, 3) uint8 RGB, got shape {tuple(shape)}")
+        h, w = int(shape[0]), int(shape[1])
+        return (h, w) + (tools.fit_plan(shape, self.width, self.height) or (h, w))
+
+    def _fit_table(self, srcs_dev, dims_dev, b, want_crops):
+        """b2o_fit_crops on the current stream: crop pointers and dims already on the device."""
+        tail = (3,) if self.color else ()
+        crnn_in = torch.empty((b, self.width, self.height) + tail, dtype=torch.float16, device=self.device)
+        crops = torch.empty((b, self.height, self.width, 3), dtype=torch.uint8, device=self.device) if want_crops else None
+        self.ctx.fit_crops(srcs_dev, dims_dev, b, crops.data_ptr() if want_crops else None, crnn_in.data_ptr(),
+                           torch.cuda.current_stream(self.device).cuda_stream)
+        return crnn_in, crops
+
+    def fit_device(self, sources, want_crops=False):
+        """tools.fit(cval=0) + the gray conversion of ``recognize`` for crops already on the GPU, in one launch.
+        ``sources``: a list of (H,W,3) uint8 CUDA tensors of any sizes, read in place.  Returns (crnn_in
+        (B,width,height[,3]) fp16, crops (B,height,width,3) u8 -- what tools.fit returns -- or None)."""
+        for s in sources:
+            if not (isinstance(s, torch.Tensor) and s.is_cuda and s.dtype == torch.uint8 and s.device == self.device):
+                raise ValueError(f"fit_device takes uint8 CUDA tensors on {self.device}")
+        sources = [s.contiguous() for s in sources]
+        b = len(sources)
+        table = np.zeros(b * 8 + b * 16, dtype=np.uint8)
+        table[: b * 8].view(np.uint64)[:] = [s.data_ptr() for s in sources]
+        table[b * 8:].view(np.int32)[:] = np.array([self._fit_dims(s.shape) for s in sources], np.int32).reshape(-1)
+        if b == 0:
+            return self._fit_table(None, None, 0, want_crops)
+        table_dev = torch.from_numpy(table).to(self.device)
+        return self._fit_table(table_dev.data_ptr(), table_dev.data_ptr() + b * 8, b, want_crops)
+
     def predict_device(self, crnn_in):
         """CRNN + greedy CTC.  crnn_in: (B,width,height) fp16 -> labels (B,steps) int32 (-1 padded); (B,200,31) -> (B,48)
         by default."""
@@ -236,6 +269,112 @@ class Recognizer:
         if not self.color and image.ndim == 3 and image.shape[-1] == 3:      # recognition.py:481-483
             image = cv2.cvtColor(image, code=cv2.COLOR_RGB2GRAY)
         return self.recognize_crops(np.ascontiguousarray(image.reshape((1, self.height, self.width) + ((3,) if self.color else ()))))[0]
+
+    def recognize_batch(self, images, chunk=1024) -> typing.List[str]:
+        """``[self.recognize(image) for image in images]`` for many pre-cropped images of any sizes, with the fit and
+        the gray conversion on the GPU (``b2o_fit_crops``) and the CRNN run over ``chunk`` crops at a time.
+
+        ``images``: a list of (H,W,3) uint8 RGB arrays, image paths (read with tools.read like ``recognize``) or
+        (H,W,3) uint8 CUDA tensors (read in place, no copy), or one (N,H,W,3) uint8 array of equally sized crops.
+        Host crops of a chunk are packed into a pinned staging buffer and sent with one host-to-device copy on a
+        side stream; two buffers alternate, so chunk k+1 is read, packed and copied while chunk k runs, and the
+        labels of chunk k are decoded once chunk k+1 is queued.  ``chunk`` bounds the CRNN workspace (about 9.5 MB
+        per crop at 31 x 200).  A crop tools.fit cannot fit raises what ``recognize`` raises (ZeroDivisionError,
+        cv2.error) before its chunk is queued; crops given as arrays or tensors are all checked before any work."""
+        if isinstance(images, np.ndarray) and images.ndim != 4:
+            raise ValueError("an array of crops must be (N, H, W, 3) uint8")
+        if isinstance(chunk, bool) or not isinstance(chunk, (int, np.integer)) or chunk < 1:
+            raise ValueError(f"chunk must be a positive integer, got {chunk!r}")
+        n = len(images)
+        if n == 0:
+            return []
+        if isinstance(images, np.ndarray):
+            self._check_host_crop(images[0])
+            dims = [self._fit_dims(images.shape[1:])] * n
+        else:
+            images = list(images)
+            dims = [None if isinstance(im, str) else self._fit_dims(self._check_device_crop(im).shape) for im in images]
+        stream = torch.cuda.current_stream(self.device)
+        if getattr(self, "_copy_stream", None) is None:
+            self._copy_stream = torch.cuda.Stream(self.device)
+            self._staging = [{"host": None, "dev": None, "labels": None, "copied": None, "fitted": None} for _ in range(2)]
+        out, pending = [], None
+        for k, start in enumerate(range(0, n, chunk)):
+            slot = self._staging[k % 2]
+            b = min(chunk, n - start)
+            crops = [self._check_device_crop(tools.read(c) if isinstance(c, str) else c) for c in images[start:start + b]]
+            cdims = [d if d is not None else self._fit_dims(c.shape) for c, d in zip(crops, dims[start:start + b])]
+            head = b * 24
+            offsets, nbytes = [], (head + 15) // 16 * 16
+            for c in crops:
+                offsets.append(None if isinstance(c, torch.Tensor) and c.is_cuda else nbytes)
+                if offsets[-1] is not None:
+                    nbytes += c.shape[0] * c.shape[1] * 3
+            if slot["copied"] is not None:
+                slot["copied"].synchronize()                  # chunk k-2's copy out of this host buffer is done
+            if slot["host"] is None or slot["host"].numel() < nbytes:
+                size = max(nbytes, nbytes * 5 // 4)
+                slot["host"] = torch.empty(size, dtype=torch.uint8, pin_memory=True)
+                with torch.cuda.stream(stream):
+                    slot["dev"] = torch.empty(size, dtype=torch.uint8, device=self.device)
+                slot["dev"].record_stream(self._copy_stream)
+                self._copy_stream.wait_stream(stream)         # the new block may still be in use by queued kernels
+            host = slot["host"].numpy()
+            base = slot["dev"].data_ptr()
+            ptrs = host[: b * 8].view(np.uint64)
+            for i, (c, off) in enumerate(zip(crops, offsets)):
+                if off is None:
+                    c = c.contiguous()
+                    crops[i] = c                              # keep a contiguous copy alive until the launch
+                    ptrs[i] = c.data_ptr()
+                else:
+                    host[off:off + c.size].reshape(c.shape)[...] = c
+                    ptrs[i] = base + off
+            host[b * 8:head].view(np.int32)[:] = np.asarray(cdims, np.int32).reshape(-1)
+            with torch.cuda.stream(self._copy_stream):
+                if slot["fitted"] is not None:
+                    self._copy_stream.wait_event(slot["fitted"])   # chunk k-2 has read this device buffer
+                slot["dev"][:nbytes].copy_(slot["host"][:nbytes], non_blocking=True)
+                slot["copied"] = torch.cuda.Event()
+                slot["copied"].record(self._copy_stream)
+            stream.wait_event(slot["copied"])
+            with torch.cuda.stream(stream):
+                crnn_in, _ = self._fit_table(base, base + b * 8, b, False)
+                slot["fitted"] = torch.cuda.Event()
+                slot["fitted"].record(stream)
+                labels = self.predict_device(crnn_in)
+                if slot["labels"] is None or slot["labels"].shape[0] < b:
+                    slot["labels"] = torch.empty((max(b, chunk), self.steps), dtype=torch.int32, pin_memory=True)
+                host_labels = slot["labels"][:b]
+                host_labels.copy_(labels, non_blocking=True)
+                ready = torch.cuda.Event()
+                ready.record(stream)
+            if pending is not None:
+                out.extend(self._decode(*pending))
+            pending = (ready, host_labels)
+        out.extend(self._decode(*pending))
+        return out
+
+    def _decode(self, ready, host_labels):
+        ready.synchronize()
+        return labels_to_text(host_labels.numpy(), self.alphabet)
+
+    @staticmethod
+    def _check_host_crop(image):
+        """A crop recognize_batch accepts: a (H,W,3) uint8 ndarray or tensor; CPU tensors come back as arrays."""
+        if isinstance(image, torch.Tensor):
+            ok = image.dtype == torch.uint8
+            image = image if image.is_cuda else image.numpy()
+        else:
+            ok = isinstance(image, np.ndarray) and image.dtype == np.uint8
+        if not ok or image.ndim != 3 or image.shape[2] != 3:
+            raise ValueError("recognize_batch takes (H, W, 3) uint8 RGB crops, paths or CUDA tensors")
+        return image
+
+    def _check_device_crop(self, image):
+        if isinstance(image, torch.Tensor) and image.is_cuda and image.device != self.device:
+            raise ValueError(f"CUDA crops must be on {self.device}, got {image.device}")
+        return self._check_host_crop(image)
 
     def recognize_from_boxes_device(self, images_t, boxes, counts, gray=None, flat=None, image_index=None):
         """images_t (N,H,W,3) u8 CUDA; boxes (N,M,4,2) f32 CUDA; counts host ndarray -> labels (B,steps) i32 CUDA.

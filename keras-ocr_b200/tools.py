@@ -75,23 +75,42 @@ def adjust_boxes(boxes, scale=1, boxes_format="boxes"):
     raise NotImplementedError(f"Unsupported boxes format: {boxes_format}")
 
 
-def fit(image, width, height, cval=255, mode="letterbox", return_scale=False):
-    """tools.fit (reference tools.py:402-452): scale the image to fit ``width`` x ``height`` keeping
-    its aspect ratio, then letterbox (pad bottom/right with ``cval``) or crop.  Host-side like the
-    reference: it only serves the single-crop ``Recognizer.recognize`` API, which is off the hot path."""
-    import cv2
-
-    sx, sy = width / image.shape[1], height / image.shape[0]
+def fit_plan(shape, width, height, mode="letterbox"):
+    """The cv2.resize size tools.fit (reference tools.py:402-452) picks for an image of ``shape``: None when it returns
+    the image unchanged (it already is ``height`` x ``width``), else ``(new_h, new_w)``.  Python floats as upstream:
+    ``sx = width / w``, ``sy = height / h``, letterbox scales by the width when ``sx <= sy`` (crop when ``sx >= sy``),
+    the other side is truncated with ``int()``.  Raises what ``fit`` raises: ZeroDivisionError for an image without
+    rows or columns, cv2.error when a resized side would be 0 (e.g. 1 x 1000 into 31 x 200).  ``fit`` and the batched
+    GPU fit (``Recognizer.recognize_batch``, ``b2o_fit_crops``) both follow this plan."""
+    h, w = int(shape[0]), int(shape[1])
+    sx, sy = width / w, height / h
     if sx == 1 and sy == 1:
-        return (image, 1) if return_scale else image
+        return None
     if mode not in ("letterbox", "crop"):
         raise NotImplementedError(f"Unsupported mode: {mode}")
     use_width = (sx <= sy) if mode == "letterbox" else (sx >= sy)
-    if use_width:
-        scale, new_w, new_h = sx, width, sx * image.shape[0]
-    else:
-        scale, new_h, new_w = sy, height, sy * image.shape[1]
-    resized = cv2.resize(image, dsize=(int(new_w), int(new_h)))
+    new_h, new_w = (int(sx * h), width) if use_width else (height, int(sy * w))
+    if new_h <= 0 or new_w <= 0:
+        import cv2
+
+        raise cv2.error(f"tools.fit: {h} x {w} resized to {new_h} x {new_w}; cv2.resize needs a non-empty size")
+    return new_h, new_w
+
+
+def fit(image, width, height, cval=255, mode="letterbox", return_scale=False):
+    """tools.fit (reference tools.py:402-452): scale the image to fit ``width`` x ``height`` keeping
+    its aspect ratio, then letterbox (pad bottom/right with ``cval``) or crop.  Host-side like the
+    reference; the size comes from ``fit_plan``.  ``Recognizer.recognize`` uses it for one crop; bulk
+    recognition (``Recognizer.recognize_batch``) runs the same plan on the GPU with ``b2o_fit_crops``."""
+    import cv2
+
+    plan = fit_plan(image.shape, width, height, mode)
+    if plan is None:
+        return (image, 1) if return_scale else image
+    sx, sy = width / image.shape[1], height / image.shape[0]
+    scale = min(sx, sy) if mode == "letterbox" else max(sx, sy)
+    new_h, new_w = plan
+    resized = cv2.resize(image, dsize=(new_w, new_h))
     if mode == "letterbox":
         fitted = np.zeros((height, width, 3), dtype="uint8") + cval
         fitted[: resized.shape[0], : resized.shape[1]] = resized[:height, :width]
